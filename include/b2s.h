@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define B2S_ABI_VERSION 2
+#define B2S_ABI_VERSION 3
 #define B2S_IDX_BITS 22
 #define B2S_IDX_MASK ((1u << B2S_IDX_BITS) - 1u)
 #define B2S_NONE_KEY 0xFFFFFFFFu
@@ -327,6 +327,116 @@ int b2s_ransac_winner_batched(const float* corr, const int32_t* c_off, const int
                               int H, double th2, const double* th2_per_pair, int32_t* best_h, int32_t* best_count,
                               uint8_t* inlier_mask, void* workspace, size_t workspace_bytes, int32_t* counts_out,
                               int32_t* n_finished_out, const b2s_record_sink* sink, int mask_stride, void* stream);
+
+/* ---- robust pose: essential / homography model selection with stability gates ------------------------
+ * The batched form of RobustPoseEstimator.estimate_pose (robust_pose_estimator.py:89-251): adaptive threshold,
+ * both RANSAC branches, per-branch inlier ratio, median parallax, cheirality and score, model selection (the
+ * essential model wins ties) and the five stability gates.  The RANSAC stages are the existing entry points
+ * (K4 / K3 / select with th2_per_pair, K7 refit + decomposition, K5 / K6 / select at th = 3); the three
+ * entry points below are the pieces around them.
+ *
+ * Configuration: the fields of RobustPoseEstimatorConfig (robust_pose_estimator.py:42-70).  Passed as a DEVICE
+ * array of n_cfg entries; pair p uses cfg[n_cfg == 1 ? 0 : p]. */
+typedef struct b2s_robust_pose_config {
+  int32_t min_matches;
+  int32_t min_inliers;
+  int32_t min_cheirality_inliers;
+  int32_t reserved;
+  double base_ransac_threshold;
+  double min_ransac_threshold;
+  double max_ransac_threshold;
+  double min_inlier_ratio;
+  double homography_bias;
+  double essential_bias;
+  double min_parallax;
+  double min_cheirality_ratio;
+} b2s_robust_pose_config;
+#define B2S_ROBUST_POSE_CONFIG_BYTES 80
+
+/* outcome of one pair: what estimate_pose returns or raises */
+#define B2S_POSE_ESTIMATE 0           /* PoseEstimate */
+#define B2S_POSE_GATE_FAILED 1        /* PoseEstimationFailure(gate reason, "relocalize", metrics) */
+#define B2S_POSE_ERR_MATCHES 2        /* ValueError: fewer than min_matches correspondences */
+#define B2S_POSE_ERR_EIGHT 3          /* ValueError: fewer than eight correspondences (ransac_essential) */
+#define B2S_POSE_ERR_ESSENTIAL 4      /* RuntimeError: essential branch (< 8 RANSAC inliers / decomposition) */
+#define B2S_POSE_ERR_HOMOGRAPHY 5     /* RuntimeError: homography branch (< 4 RANSAC inliers / decomposition) */
+#define B2S_POSE_ERR_TRANSLATION 6    /* ValueError: zero translation; `method` names the branch */
+/* method */
+#define B2S_POSE_METHOD_ESSENTIAL 0
+#define B2S_POSE_METHOD_HOMOGRAPHY 1
+/* gate: the first failed stability gate, in the reference's order */
+#define B2S_GATE_NONE 0
+#define B2S_GATE_LOW_INLIER_COUNT 1
+#define B2S_GATE_LOW_INLIER_RATIO 2
+#define B2S_GATE_LOW_PARALLAX 3
+#define B2S_GATE_CHEIRALITY_INLIERS 4
+#define B2S_GATE_CHEIRALITY_RATIO 5
+
+/* One fixed-size result per pair.  The diagnostics are those of the selected model (of the failing branch for
+ * an error); e_* / h_* are the two RANSAC winners (hypothesis index, inlier count; -1 when the branch did not
+ * run), which is what a caller needs to leave seeded generators where the reference leaves them.
+ * median_parallax is the float32 median widened to float64; t is normalised. */
+typedef struct b2s_pose_result {
+  int32_t outcome;
+  int32_t method;
+  int32_t gate;
+  int32_t match_count;
+  int32_t inliers;
+  int32_t cheirality_inliers;
+  int32_t e_best_h;
+  int32_t e_inliers;
+  int32_t h_best_h;
+  int32_t h_inliers;
+  int32_t reserved[2];
+  double inlier_ratio;
+  double median_parallax;
+  double cheirality_ratio;
+  double score;
+  double score_essential;
+  double score_homography;
+  double threshold;
+  double R[9];
+  double t[3];
+} b2s_pose_result;
+#define B2S_POSE_RESULT_BYTES 200
+#ifdef __cplusplus
+static_assert(sizeof(b2s_robust_pose_config) == B2S_ROBUST_POSE_CONFIG_BYTES, "b2s_robust_pose_config layout");
+static_assert(sizeof(b2s_pose_result) == B2S_POSE_RESULT_BYTES, "b2s_pose_result layout");
+#else
+_Static_assert(sizeof(b2s_robust_pose_config) == B2S_ROBUST_POSE_CONFIG_BYTES, "b2s_robust_pose_config layout");
+_Static_assert(sizeof(b2s_pose_result) == B2S_POSE_RESULT_BYTES, "b2s_pose_result layout");
+#endif
+
+/* Median displacement per pair: np.median(np.linalg.norm(pts2[sel] - pts1[sel], axis=1)) on the float32
+ * correspondences, bit for bit (float32 norm without contraction, exact radix select on the bit patterns,
+ * float32(a + b) / 2 for an even count, 0 for an empty selection; a NaN displacement gives NaN).  mask NULL =
+ * all correspondences.  cfg (device, n_cfg entries) non-NULL: also the adaptive threshold of
+ * adaptive_ransac_threshold (feature_pipeline.py.bak:114-129) in float64, th_out and th2_out = th * th
+ * (either may be NULL).  One CTA per pair; any count. */
+int b2s_displacement_median_batched(const float* corr, const int32_t* c_off, const int32_t* c_count, const uint8_t* mask,
+                                    int n_pairs, const b2s_robust_pose_config* cfg, int n_cfg, float* median_out,
+                                    double* th_out, double* th2_out, void* stream);
+
+/* n-point normalised DLT of each pair's masked correspondences (dlt_homography, homography.py:118-142, the
+ * final refit of ransac_homography :216): Hartley normalisation, Gram matrix in float64 reduced in a fixed order,
+ * eigenvector of its smallest eigenvalue, de-normalised with H[2][2] = 1.  H_out [pair][9] (zeros when fewer
+ * than 4 correspondences take part); n_used (optional) = correspondences that took part. */
+int b2s_refit_homography_batched(const float* corr, const int32_t* c_off, const int32_t* c_count, const uint8_t* mask,
+                                 int n_pairs, double* H_out, int32_t* n_used, void* stream);
+
+/* Decision stage: per pair the essential branch (e_best_h / e_inliers from b2s_ransac_select, e_R / e_t from
+ * b2s_pose_pick, e_votes from b2s_decompose_essential_batched, e_median = inlier median), the homography branch
+ * (h_best_h / h_inliers from b2s_homography_select, H_fit from b2s_refit_homography_batched, decompose_homography
+ * homography.py:59-78), all_median / th from b2s_displacement_median_batched; model selection and gates.
+ * results [n_pairs]; out_mask [c_off[p] .. + c_count[p]) = the selected model's inlier flags (also for a gate
+ * failure; zero for an error outcome); mask_stride > 0: out_mask[c_off[p] + c_count[p] .. c_off[p] + mask_stride)
+ * is zeroed too (the unused tail of a compact slot).  Kinv_host: HOST 3x3 row-major (NULL = identity). */
+int b2s_robust_pose_decide(const int32_t* c_off, const int32_t* c_count, int n_pairs, const int32_t* e_best_h,
+                           const int32_t* e_inliers, const uint8_t* e_mask, const double* e_R, const double* e_t,
+                           const int32_t* e_votes, const float* e_median, const float* all_median, const double* th,
+                           const int32_t* h_best_h, const int32_t* h_inliers, const uint8_t* h_mask, const double* H_fit,
+                           const double* Kinv_host, const b2s_robust_pose_config* cfg, int n_cfg,
+                           b2s_pose_result* results, uint8_t* out_mask, int mask_stride, void* stream);
 
 /* ---- measurement helper ----------------------------------------------------------
  * Saturates one SM pipe with independent instructions to measure its rate:

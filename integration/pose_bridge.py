@@ -500,6 +500,115 @@ class RobustPoseEstimator:
         diag = PoseEstimationDiagnostics("homography", len(pts1), len(inliers), ratio, parallax, len(inliers), 1.0, score)
         return PoseEstimate(R, _normalize_translation(t), inliers, diag)
 
+    def estimate_pose_batch(self, kp1_list, kp2_list, matches_list, intrinsics: np.ndarray, rngs=None,
+                            seed: int | None = None, configs=None) -> list:
+        """``estimate_pose`` for many pairs in one pass on the device -> one entry per pair: the PoseEstimate the
+        single call returns, or the exception instance it would raise (same type and message; for
+        PoseEstimationFailure the same reason, recovery action and metrics).
+
+        The argument checks run on the host: a bad ``intrinsics`` shape fails the whole call; a pair with fewer than
+        ``min_matches`` matches, empty keypoints or fewer than eight correspondences gets its ValueError and never
+        reaches the device (a batch of such pairs needs no CUDA).  All other pairs go through ONE
+        ``b200slam.robust_pose.RobustPose.run``: one upload, one download.
+
+        rngs: optional ``(essential_rng, homography_rng)`` per pair; the samples are drawn from them exactly as the
+        reference's loops draw them and each generator is left where the single call leaves it (the homography
+        generator untouched when the essential branch raises).  With ``rngs=None`` and ``RNG_FACTORY`` set, two
+        generators are requested per pair that reaches RANSAC, in pair order, essential first — the order of
+        consecutive single calls whenever no essential branch raises (a single call that raises there never asks
+        for its homography generator).  Otherwise the device sampler draws with ``seed`` (random when None).
+        configs: optional per-pair RobustPoseEstimatorConfig (default: this estimator's for every pair)."""
+        if intrinsics.shape != (3, 3):
+            raise ValueError("Intrinsics must be a 3x3 matrix")
+        n_pairs = len(matches_list)
+        if not (len(kp1_list) == len(kp2_list) == n_pairs):
+            raise ValueError("kp1_list, kp2_list and matches_list differ in length")
+        cfgs = [self.config] * n_pairs if configs is None else list(configs)
+        if len(cfgs) != n_pairs:
+            raise ValueError("one config per pair")
+        out: list = [None] * n_pairs
+        live, pts = [], []
+        for p in range(n_pairs):
+            kp1, kp2, matches = kp1_list[p], kp2_list[p], matches_list[p]
+            if len(matches) < cfgs[p].min_matches:
+                out[p] = ValueError("Not enough matches for pose estimation")
+            elif not kp1 or not kp2:
+                out[p] = ValueError("Keypoints must be non-empty")
+            elif len(matches) < 8:                                   # ransac_essential's own check (homography.py:305)
+                out[p] = ValueError("At least eight correspondences are required")
+            else:
+                live.append(p)
+                pts.append(matches_to_points(kp1, kp2, matches))
+        if not live:
+            return out
+        from b200slam import _capi
+
+        torch = _capi.require_cuda()
+        from b200slam import robust_pose as rp
+
+        max_iter = 2000
+        L = len(live)
+        counts = np.array([len(a) for a, _ in pts], np.int32)
+        off = np.zeros(L + 1, np.int32)
+        np.cumsum(counts, out=off[1:])
+        rows = int(off[-1])
+        if rngs is None and RNG_FACTORY is not None:
+            gens = [(RNG_FACTORY(), RNG_FACTORY()) for _ in live]
+        elif rngs is not None:
+            gens = [tuple(rngs[p]) for p in live]
+        else:
+            gens = None
+        # one host buffer, one upload: corr (float32 bits) | c_off | c_count | samples_e | samples_h
+        n_smp = L * max_iter * 12 if gens is not None else 0
+        host = np.zeros(rows * 4 + (L + 1) + L + n_smp, np.int32)
+        corr = host[:rows * 4].view(np.float32).reshape(rows, 4)
+        for i, (a, b) in enumerate(pts):
+            corr[off[i]:off[i + 1], :2] = a
+            corr[off[i]:off[i + 1], 2:] = b
+        host[rows * 4:rows * 4 + L + 1] = off
+        host[rows * 4 + L + 1:rows * 4 + 2 * L + 1] = counts
+        states = []
+        if gens is not None:
+            base = rows * 4 + 2 * L + 1
+            se = host[base:base + L * max_iter * 8].reshape(L, max_iter, 8)
+            sh = host[base + L * max_iter * 8:base + n_smp].reshape(L, max_iter, 4)
+            for i, (ge, gh) in enumerate(gens):                     # homography.py:325 and :193, the same streams
+                se[i], st_e = _draw_reference_stream(ge, int(counts[i]), 8, max_iter)
+                sh[i], st_h = _draw_reference_stream(gh, int(counts[i]), 4, max_iter)
+                states.append((st_e, st_h))
+        if seed is None:
+            seed = int(np.random.SeedSequence().entropy & (2 ** 63 - 1))
+        dev = torch.device("cuda", torch.cuda.current_device())
+        d = torch.from_numpy(host).to(dev)
+        corr_d = d[:rows * 4].view(torch.float32).view(max(rows, 0), 4)
+        off_d, cnt_d = d[rows * 4:rows * 4 + L + 1], d[rows * 4 + L + 1:rows * 4 + 2 * L + 1]
+        smp_e = smp_h = None
+        if gens is not None:
+            base = rows * 4 + 2 * L + 1
+            smp_e = d[base:base + L * max_iter * 8].view(L, max_iter, 8)
+            smp_h = d[base + L * max_iter * 8:base + n_smp].view(L, max_iter, 4)
+        if not hasattr(self, "_device"):
+            self._device = rp.RobustPose()
+        cfg_live = cfgs[0] if configs is None else [cfgs[p] for p in live]
+        res = self._device.run(corr_d, off_d, cnt_d, L, intrinsics, cfg_live, samples_e=smp_e, samples_h=smp_h, seed=seed,
+                               max_m=int(counts.max()), hypotheses=max_iter)
+        packed = res.packed.cpu().numpy()                            # the one download
+        recs = rp.decode_results(packed[:L * rp.POSE_RESULT_BYTES])
+        mask = packed[L * rp.POSE_RESULT_BYTES:]
+        for i, p in enumerate(live):
+            r = recs[i]
+            out[p] = decode_pose_result(r, np.flatnonzero(mask[off[i]:off[i + 1]]))
+            if gens is not None:
+                n = int(counts[i])
+                (ge, gh), (st_e, st_h) = gens[i], states[i]
+                if int(r["e_best_h"]) >= 0 and r["e_inliers"] > 0.8 * n:   # the loop stopped early (homography.py:338)
+                    _rewind_to_reference_state(ge, st_e, n, 8, int(r["e_best_h"]) + 1)
+                if not _homography_ran(r):
+                    _rewind_to_reference_state(gh, st_h, n, 4, 0)
+                elif int(r["h_best_h"]) >= 0 and r["h_inliers"] > 0.8 * n:
+                    _rewind_to_reference_state(gh, st_h, n, 4, int(r["h_best_h"]) + 1)
+        return out
+
     def _apply_stability_gates(self, est: PoseEstimate) -> None:
         cfg, d = self.config, est.diagnostics
         metrics = {"match_count": float(d.match_count), "inliers": float(d.inliers),
@@ -516,6 +625,47 @@ class RobustPoseEstimator:
                 raise PoseEstimationFailure("cheirality_inliers", "relocalize", metrics)
             if d.cheirality_ratio < cfg.min_cheirality_ratio:
                 raise PoseEstimationFailure("cheirality_ratio", "relocalize", metrics)
+
+
+def _homography_ran(r) -> bool:
+    """estimate_pose reaches ransac_homography unless the essential branch raised first."""
+    from b200slam import robust_pose as rp
+
+    o = int(r["outcome"])
+    if o in (rp.POSE_ERR_MATCHES, rp.POSE_ERR_EIGHT, rp.POSE_ERR_ESSENTIAL):
+        return False
+    return not (o == rp.POSE_ERR_TRANSLATION and int(r["method"]) == 0)
+
+
+def decode_pose_result(r, inlier_indices: np.ndarray):
+    """One b2s_pose_result (a record of b200slam.robust_pose.POSE_RESULT_DTYPE) -> what estimate_pose returns
+    (PoseEstimate) or the exception instance it raises, with the single call's messages.  inlier_indices: the
+    selected model's inliers (flatnonzero of the pair's mask)."""
+    from b200slam import robust_pose as rp
+
+    o = int(r["outcome"])
+    if o == rp.POSE_ERR_MATCHES:
+        return ValueError("Not enough matches for pose estimation")
+    if o == rp.POSE_ERR_EIGHT:
+        return ValueError("At least eight correspondences are required")
+    if o == rp.POSE_ERR_ESSENTIAL:
+        return RuntimeError("Essential matrix pose estimation failed")
+    if o == rp.POSE_ERR_HOMOGRAPHY:
+        return RuntimeError("Homography pose estimation failed")
+    if o == rp.POSE_ERR_TRANSLATION:
+        return ValueError("Translation norm is zero")
+    if o not in (rp.POSE_ESTIMATE, rp.POSE_GATE_FAILED):
+        raise ValueError(f"unknown pose result outcome {o}")
+    diag = PoseEstimationDiagnostics(rp.METHODS[int(r["method"])], int(r["match_count"]), int(r["inliers"]),
+                                     float(r["inlier_ratio"]), float(r["median_parallax"]), int(r["cheirality_inliers"]),
+                                     float(r["cheirality_ratio"]), float(r["score"]))
+    if o == rp.POSE_GATE_FAILED:
+        metrics = {"match_count": float(diag.match_count), "inliers": float(diag.inliers),
+                   "inlier_ratio": float(diag.inlier_ratio), "median_parallax": float(diag.median_parallax),
+                   "cheirality_ratio": float(diag.cheirality_ratio), "cheirality_inliers": float(diag.cheirality_inliers)}
+        return PoseEstimationFailure(rp.GATE_REASONS[int(r["gate"])], "relocalize", metrics)
+    return PoseEstimate(np.array(r["R"], dtype=np.float64).reshape(3, 3), np.array(r["t"], dtype=np.float64),
+                        np.asarray(inlier_indices, dtype=np.int64), diag)
 
 
 # --------------------------------------------------------------------------- #

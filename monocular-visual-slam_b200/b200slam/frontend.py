@@ -664,6 +664,9 @@ class FrontendConfig:
                                # scoring (0.35 ms).  Same counts.
     winner_only: bool = False  # True: same winner / inlier mask, but hypotheses that cannot win are abandoned early
                                # (EssentialRansac.winner); FrontendResult.counts is then None
+    robust_pose: "RobustPoseConfig | None" = None   # set: RobustPoseEstimator.estimate_pose for every pair (robust_pose.py):
+                               # the essential RANSAC runs at the adaptive per-pair threshold, the homography branch,
+                               # model selection and gates follow; FrontendResult.robust / robust_mask hold the answer
 
 
 @dataclass
@@ -680,6 +683,8 @@ class FrontendResult:
     t: "torch.Tensor | None" = None
     votes: "torch.Tensor | None" = None
     records: "torch.Tensor | None" = None
+    robust: "torch.Tensor | None" = None        # uint8 [n_pairs, 200] b2s_pose_result (robust_pose.decode_results)
+    robust_mask: "torch.Tensor | None" = None   # the selected model's inlier flags, layout of inlier_mask
 
 
 class Frontend:
@@ -690,6 +695,7 @@ class Frontend:
         self.matcher = HammingMatcher(variant=variant, t_split=t_split)
         self.ransac = EssentialRansac()
         self.pose = None
+        self.robust = None
         self.launches_per_run = 0
 
     def score(self, sel: Selection, b: PairBatch, E):
@@ -709,12 +715,30 @@ class Frontend:
         before the record kernel — where ShardedFrontend starts and joins the collective of the PREVIOUS batch, so
         that it overlaps the multi-wave RANSAC kernels and never the persistent one-CTA-per-SM Hamming kernel."""
         c = self.cfg
+        if c.robust_pose is not None:
+            if records is not None or pair_id0 != 0:
+                raise ValueError("robust_pose does not write result records and takes no pair_id0 offset yet")
+            if c.winner_only or c.scoring == "tc":
+                raise ValueError("robust_pose scores with the CUDA-core kernel (scoring='cuda', winner_only=False)")
         keys = self.matcher.knn2(b, need_second=bool(c.use_ratio))
         sel = self.matcher.select(b, keys, use_ratio=c.use_ratio, use_cross=c.use_cross, ratio=c.ratio,
                                   sort_by_distance=True, max_matches=c.max_matches, with_corr=True,
                                   compact=True)
         if after_select is not None:
             after_select()
+        if c.robust_pose is not None:
+            if self.robust is None:
+                from .robust_pose import RobustPose
+
+                self.robust = RobustPose()
+            out = self.robust.run(sel.corr, sel.c_off, sel.count, b.n_pairs, K, c.robust_pose, samples_e=samples, seed=c.seed,
+                                  max_m=sel.stride or b.max_nq, hypotheses=c.hypotheses, precision=c.precision,
+                                  mask_stride=sel.stride)
+            if before_records is not None:
+                before_records()
+            return FrontendResult(keys, sel, out.E, out.counts, out.best_h, out.best_count, out.inlier_mask,
+                                  E_refit=out.E_refit, R=out.R, t=out.t, votes=out.votes, robust=out.results,
+                                  robust_mask=out.mask)
         E = self.ransac.hypotheses(sel.corr, sel.c_off, sel.count, b.n_pairs, c.hypotheses,
                                    samples=samples, seed=c.seed, K=K, pair_id0=pair_id0)
         th2 = c.threshold ** 2
