@@ -42,9 +42,12 @@ def test_dlt_hypotheses_and_scores_match_reference(hgold, R):
         Href = torch.from_numpy(np.nan_to_num(Hs).reshape(1, -1, 9).copy()).cuda()
         counts = R.score(corr, off, cnt, 1, Href, th).cpu().numpy()[0]
         np.testing.assert_array_equal(counts[valid], masks[valid].sum(1), err_msg=name)
-        # device hypotheses: counts within the flip tolerance of the reference's
+        # device hypotheses: counts equal the high-precision reference's on the same hypotheses outside the band
         c_dev = R.score(corr, off, cnt, 1, Hm, th).cpu().numpy()[0]
-        assert np.abs(c_dev[valid] - masks[valid].sum(1)).max() <= max(1, FLIP_TOL * len(src)), name
+        ref, band = hom.classify(Hd, src, dst, th)
+        n_band = hom.check_counts(c_dev, ref, band, name)
+        print(f"{name}: band cases excused {n_band}")
+        assert n_band == 0, name
         best_h, best_c, mask = R.select(torch.from_numpy(counts[None].astype(np.int32)).cuda(), corr, off, cnt, 1, Href, th)
         full = np.where(valid, masks.sum(1), 0)
         want = hom.select_hypothesis(np.where(valid, counts, 0), len(src))
@@ -98,6 +101,8 @@ def test_device_sampler_ragged_and_degenerate(R):
             continue
         assert all(len(set(r)) == 4 and 0 <= min(r) and max(r) < m for r in smp[p])
         s, d = srcs[p]
-        _, oc = hom.score_hypotheses(Hm[p].cpu().numpy().reshape(-1, 3, 3), s, d, 3.0)
-        assert np.abs(oc - counts[p]).max() <= 1
+        ref, band = hom.classify(Hm[p].cpu().numpy().reshape(-1, 3, 3), s, d, 3.0)
+        n_band = hom.check_counts(counts[p], ref, band, f"M={m}")
+        print(f"M={m}: band cases excused {n_band}")
+        assert n_band == 0
         assert best_c[p] >= 0.9 * m                                                            # the planted similarity is found
