@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define B2S_ABI_VERSION 3
+#define B2S_ABI_VERSION 4
 #define B2S_IDX_BITS 22
 #define B2S_IDX_MASK ((1u << B2S_IDX_BITS) - 1u)
 #define B2S_NONE_KEY 0xFFFFFFFFu
@@ -240,7 +240,7 @@ int b2s_hamming_knn2_shared(const uint8_t* desc, const int32_t* blk_row0, const 
                             uint32_t* fwd_second, uint32_t* bwd_best, int t_split, int need_second, void* workspace,
                             size_t workspace_bytes, void* stream);
 /* Diagnostics: work decomposition of the most recent single-product launch — query sub-tiles per
- * work item (2 or 4), train-axis split, CTAs. */
+ * work item (always 2), train-axis split, CTAs. */
 void b2s_hamming_last_plan(int* subs, int* t_split, int* grid);
 
 /* K9 — bag-of-words candidate ranking, the step in front of the relocalizer's matching (next-row #4).
@@ -446,15 +446,6 @@ int b2s_robust_pose_decide(const int32_t* c_off, const int32_t* c_count, int n_p
  * thread; *ops_out = total thread-level instructions executed (the caller times it). */
 int b2s_pipe_microbench(int which, int iters, int ctas_per_sm, double* ops_out, uint32_t* sink,
                         void* stream);
-
-/* Diagnostics: when dev_buf != NULL (device memory, 8 x uint64 per SM) the i8 Hamming kernel
- * records, per CTA, clock64 totals: [0] MMA thread total, [1] MMA waiting for a free TMEM stage,
- * [2] MMA waiting for operand tiles, [3] producer waiting for a free ring slot, [4] epilogue
- * warp total, [5] epilogue waiting for accumulators, [6] tile pairs.  NULL switches it off.
- * mode (results become meaningless, timing only): bit 0 = the epilogue drains nothing,
- * bit 1 = the operand ring is loaded once and then reused.  Bits that keep the results exact:
- * 16 = the 32x32b A/B epilogue, 32 / 64 = force 2 / 4 query sub-tiles per work item.  0 = normal. */
-void b2s_hamming_i8_debug(unsigned long long* dev_buf, int mode);
 
 /* Measurement: enable = 1 / 0 switches a CUDA-event pair around the tcgen05 Hamming kernel
  * proper (without the operand pre-pass) on and off, enable < 0 leaves it as it is; if last_ms

@@ -21,7 +21,7 @@ IDX_MASK = (1 << IDX_BITS) - 1
 NONE_KEY = 0xFFFFFFFF
 DESC_BYTES = 32
 SELECT_MAX_QUERIES = 32768
-ABI_VERSION = 3
+ABI_VERSION = 4
 VARIANT_POPC = 0
 VARIANT_I8MMA = 1
 VARIANT_I8MMA1 = 2
@@ -124,8 +124,6 @@ def _declare(lib):
     lib.b2s_refit_homography_batched.argtypes = [vp, vp, vp, vp, i32, vp, vp, vp]
     lib.b2s_robust_pose_decide.restype = i32
     lib.b2s_robust_pose_decide.argtypes = [vp, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, i32, vp]
-    lib.b2s_hamming_i8_debug.restype = None
-    lib.b2s_hamming_i8_debug.argtypes = [vp, i32]
     lib.b2s_hamming_kernel_timing.restype = i32
     lib.b2s_hamming_kernel_timing.argtypes = [i32, C.POINTER(C.c_float)]
     lib.b2s_mma_microbench.restype = i32
@@ -142,7 +140,7 @@ EXPORTS = (
     "b2s_hamming_knn2_batched", "b2s_hamming_set_config", "b2s_hamming_get_config",
     "b2s_select_matches", "b2s_eight_point_batched", "b2s_ransac_score_batched",
     "b2s_ransac_select", "b2s_pipe_microbench", "b2s_mma_microbench", "b2s_tmem_microbench",
-    "b2s_hamming_i8_debug", "b2s_hamming_kernel_timing", "b2s_ransac_score_tc_workspace_bytes", "b2s_ransac_score_tc",
+    "b2s_hamming_kernel_timing", "b2s_ransac_score_tc_workspace_bytes", "b2s_ransac_score_tc",
     "b2s_homography_dlt_batched", "b2s_homography_score_batched", "b2s_homography_select", "b2s_decompose_essential_batched", "b2s_refit_essential_batched", "b2s_pose_pick", "b2s_five_point_batched",
     "b2s_bow_histogram_batched", "b2s_bow_cosine", "b2s_hamming_shared_workspace_bytes", "b2s_hamming_knn2_shared", "b2s_hamming_last_plan",
     "b2s_record_bytes", "b2s_pack_records", "b2s_rank_pairs", "b2s_ransac_winner_workspace_bytes", "b2s_ransac_winner_batched",

@@ -55,7 +55,6 @@ int hamming_i8_shared_launch(const uint8_t* desc, const int32_t* blk_row0, const
                              size_t workspace_bytes, cudaStream_t st);
 void hamming_i8_last_plan(int* subs, int* t_split, int* grid);
 
-void hamming_i8_set_debug(unsigned long long* dev_buf, int mode);
 int hamming_i8_timing(int enable, float* last_ms);
 int mma_rate_launch(int iters, int n_dim, double* macs_out, cudaStream_t st);
 int tmem_read_launch(int iters, int warps, double* bytes_out, uint32_t* sink, cudaStream_t st);
@@ -231,8 +230,6 @@ size_t b2s_hamming_workspace_bytes_v(int variant, int n_pairs, int total_nq, int
     return b2s::hamming_i8_workspace_bytes(n_pairs, total_nq, max_nq, max_nt, variant == B2S_VARIANT_I8MMA1 ? t_split : 1);
   return b2s_hamming_workspace_bytes(total_nq, t_split);
 }
-
-void b2s_hamming_i8_debug(unsigned long long* dev_buf, int mode) { b2s::hamming_i8_set_debug(dev_buf, mode); }
 
 int b2s_hamming_kernel_timing(int enable, float* last_ms) { return b2s::hamming_i8_timing(enable, last_ms); }
 

@@ -59,34 +59,25 @@ __device__ __forceinline__ uint32_t spread4(uint32_t nib, bool train) {
   return train ? (0xF8F8F8F8u - sp * 0xF0u) : (0x08080808u + sp * 0xF0u);
 }
 
-// layout 3 (shipped, 16x256b epilogue): UNIFIED tiles, 18 chunks, the same tile serves a frame as query
-// and as train operand.  Data: bit clear / set -> +8 / -8 on both sides, so the 8 data K-steps give
+// Unified tiles (single-product kernel): 18 chunks, the same tile serves a frame as query and as
+// train operand.  Data: bit clear / set -> +8 / -8 on both sides, so the 8 data K-steps give
 // 64 (256 - 2 ham) = 2^14 - 128 ham: the accumulator DEcreases with the distance.  The index K-step
 // multiplies the query tile's chunk 17 with the train tile's chunk 16:
 //     A (chunk 17) [-1, r, 127, 127, 127, 127, 2, 0..]     B (chunk 16) [c, -1, 127, 127, 127, 6, 1, 0..]
 // = -c - r + 3 * 16129 + 762 + 2 = 49151 - c - r, so that  acc = 65535 - (128 ham + c + r) = ~key:
-// the COMPLEMENT of the 16-bit key of layouts 1 / 2.  The epilogue takes maxima instead of minima
-// and complements its few results.  Padding rows are all zero on both sides: acc = 0, below every
-// real value (>= 32513), and 65535 = "none" after the complement.
-// layout 0: two-product tiles (17 chunks; index chunk [r, 64 x4, 0..], padding rows [127 x9, 0..]).
-// layout 1 / 2: single-product query / train tiles.  There the index K-step multiplies the
-// QUERY tile's own chunk 16 (A side) with the TRAIN tile's chunk 16 (B side), 14 int8 slots:
-//     A valid  [1, 64 x4, r, 0 x4, 64 x4]      B valid  [c, 64 x4, 1, 64 x4, 0 x4]
-//     A pad    [1, 127 x4, 127, 127 x4, 0 x4]  B pad    [127, 127 x4, 1, 0 x4, 127 x4]
-// valid.valid = c + r + 2^14 (cancels the data bias), valid.pad = 65151 + r, pad.valid =
-// 65151 + c: the accumulator is 128*ham + column + row for real pairs and lands in the padding
-// range (>= 0xFE00 after the row or the column is taken off again) otherwise.  Query tiles
-// carry an 18th, all-zero chunk so that the second half of the K = 32 index step multiplies
-// whatever follows the train tile's chunk 16 in shared memory by zero.
+// the COMPLEMENT of the 16-bit key 128 ham + column + row.  The epilogue takes maxima instead of
+// minima and complements its few results.  Padding rows are all zero on both sides: acc = 0, below
+// every real value (>= 32513), and 65535 = "none" after the complement.
+// Otherwise two-product tiles (17 chunks; index chunk [r, 64 x4, 0..], padding rows [127 x9, 0..]).
 __global__ void __launch_bounds__(128) expand_pm8_kernel(const uint8_t* __restrict__ desc,
                                                          const int32_t* __restrict__ off,
                                                          const int32_t* __restrict__ src, int tiles_per_pair,
-                                                         int train, int layout, uint4* __restrict__ out,
+                                                         int train, bool unified, uint4* __restrict__ out,
                                                          const int32_t* __restrict__ blk_rows,
                                                          const int32_t* __restrict__ blk_tile0) {
   // one CTA per (tile, pair), one thread per row: the row's 32 bytes are read once (2 x LDG.128)
   // and its 17 / 18 k-chunks leave as STG.128 that are contiguous across the 128 threads.
-  const int chunks = (layout == 1 || layout == 3) ? kI8Chunks + 1 : kI8Chunks;
+  const int chunks = unified ? kI8Chunks + 1 : kI8Chunks;
   const int pair = blockIdx.y, tile = blockIdx.x, r = threadIdx.x;
   // block mode (blk_rows != nullptr): "pair" is a descriptor BLOCK (a frame) shared by several pairs:
   // blk_rows[b] rows starting at input row src[b], expanded once to tiles blk_tile0[b] ...
@@ -110,7 +101,7 @@ __global__ void __launch_bounds__(128) expand_pm8_kernel(const uint8_t* __restri
     uint4 v = make_uint4(0, 0, 0, 0);
     if (valid) {
       const uint32_t bits = (w[kc >> 1] >> (16 * (kc & 1))) & 0xFFFFu;   // descriptor bytes 2 kc, 2 kc + 1
-      const bool tr = train && layout != 3;   // unified tiles: one sign for both roles
+      const bool tr = train && !unified;   // unified tiles: one sign for both roles
       v.x = spread4(bits & 15u, tr);
       v.y = spread4((bits >> 4) & 15u, tr);
       v.z = spread4((bits >> 8) & 15u, tr);
@@ -118,27 +109,16 @@ __global__ void __launch_bounds__(128) expand_pm8_kernel(const uint8_t* __restri
     }
     dst[kc * kI8Tile] = v;
   }
-  uint4 v;
-  if (layout == 3) {
-    // unified tile: chunk 16 = index chunk of the row as a TRAIN row (B side; a train slot is then ONE
-    // contiguous 34 KB copy), chunk 17 = as a QUERY row (A side); padding rows are all zero.  See the 16x256b epilogue for the arithmetic.
+  if (unified) {
+    // chunk 16 = index chunk of the row as a TRAIN row (B side; a train slot is then ONE contiguous
+    // 34 KB copy), chunk 17 = as a QUERY row (A side); padding rows are all zero
     const uint32_t rr = (uint32_t)r;
     dst[17 * kI8Tile] = valid ? make_uint4(0x7F7F00FFu | (rr << 8), 0x00027F7Fu, 0u, 0u) : make_uint4(0u, 0u, 0u, 0u);
     dst[16 * kI8Tile] = valid ? make_uint4(0x7F7FFF00u | rr, 0x0001067Fu, 0u, 0u) : make_uint4(0u, 0u, 0u, 0u);
-    return;
-  }
-  if (layout == 0) {
-    v = valid ? make_uint4((uint32_t)r | 0x40404000u, 0x00000040u, 0u, 0u)     // [r, 64, 64, 64, 64, 0, ...]
-              : make_uint4(0x7F7F7F7Fu, 0x7F7F7F7Fu, 0x0000007Fu, 0u);         // [127 x9, 0, ...] -> acc = 65151
-  } else if (layout == 1) {
-    v = valid ? make_uint4(0x40404001u, 0x00000040u | ((uint32_t)r << 8), 0x40400000u, 0x00004040u)
-              : make_uint4(0x7F7F7F01u, 0x7F7F7F7Fu, 0x00007F7Fu, 0u);
   } else {
-    v = valid ? make_uint4(0x40404000u | (uint32_t)r, 0x40400140u, 0x00004040u, 0u)
-              : make_uint4(0x7F7F7F7Fu, 0x0000017Fu, 0x7F7F0000u, 0x00007F7Fu);
+    dst[16 * kI8Tile] = valid ? make_uint4((uint32_t)r | 0x40404000u, 0x00000040u, 0u, 0u)  // [r, 64, 64, 64, 64, 0, ...]
+                              : make_uint4(0x7F7F7F7Fu, 0x7F7F7F7Fu, 0x0000007Fu, 0u);      // [127 x9, 0, ...] -> acc = 65151
   }
-  dst[16 * kI8Tile] = v;
-  if (layout == 1) dst[17 * kI8Tile] = make_uint4(0, 0, 0, 0);
 }
 
 __device__ __forceinline__ void tc_mma_i8(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
@@ -270,17 +250,12 @@ struct I8Params {
   int q_tiles, t_tiles, n_pairs;
   const int32_t* __restrict__ q_xt;  // optional (shared blocks): first expanded tile of each pair's query / train side,
   const int32_t* __restrict__ t_xt;  // both in the ONE unified buffer qx == tx; nullptr = pair * q_tiles / pair * t_tiles
-  unsigned long long* dbg;  // optional per-CTA stall counters (b2s_hamming_i8_debug), else nullptr
-  int mode;                 // diagnostics only: bit 0 = epilogue does no work, bit 1 = ring is loaded once,
-                            // (single-product kernel) bit 2 = no column butterfly, bit 3 = no row top-2
   // single-product kernel only: t_split > 1 cuts every (pair, query block) into t_split work items along the
   // train axis; item `part` writes its rows' top-2 to partial[part * total_nq + row] and a merge kernel folds them
   int t_split;
   int total_nq;
   uint2* __restrict__ partial;
 };
-// dbg layout per CTA (8 x u64): [0] MMA thread total, [1] MMA wait tempty, [2] MMA wait full/qfull,
-// [3] producer wait empty, [4] epilogue warp 2 total, [5] epilogue wait tfull, [6] tile pairs, [7] -
 
 // 64 columns (32 packed registers) folded into 2 interleaved packed top-2 chains.  The low and
 // the high 16-bit lane of every register are independent streams (even / odd columns).  Two
@@ -367,7 +342,6 @@ __global__ void __launch_bounds__(kI8Threads, 1) hamming_knn2_i8_kernel(const I8
     // ===== producer =====
     if (lane == 0) {
       uint32_t n = 0, g = 0;  // items seen by this CTA, train tiles streamed by this CTA
-      long long w_empty = 0;
       for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
         const int pair = w / p.q_tiles, qt = w - pair * p.q_tiles;
         const int nq = p.q_off[pair + 1] - p.q_off[pair];
@@ -378,17 +352,12 @@ __global__ void __launch_bounds__(kI8Threads, 1) hamming_knn2_i8_kernel(const I8
         const uint8_t* tsrc = p.tx + (size_t)pair * p.t_tiles * kI8TileBytes;
         for (int t = 0; t < n_tt; ++t, ++g) {
           const uint32_t s = g % kI8Stages;
-          const long long c0 = p.dbg ? clock64() : 0;
           if (g >= kI8Stages) mbar_wait_bounded(&b_empty[s], ((g / kI8Stages) - 1u) & 1u);
-          if (p.dbg) w_empty += clock64() - c0;
           if (t == 0) {  // the item's query tile rides on the barrier of its first train tile
             if (n >= 2) mbar_wait_bounded(&b_qempty[qb], ((n >> 1) - 1u) & 1u);
             mbar_arrive_expect_tx(&b_full[s], 2 * kI8TileBytes);
             bulk_g2s(s_q + (size_t)qb * kI8TileBytes, p.qx + ((size_t)pair * p.q_tiles + qt) * kI8TileBytes,
                      kI8TileBytes, &b_full[s]);
-          } else if ((p.mode & 2) && g >= kI8Stages) {
-            mbar_arrive(&b_full[s]);
-            continue;
           } else {
             mbar_arrive_expect_tx(&b_full[s], kI8TileBytes);
           }
@@ -396,15 +365,12 @@ __global__ void __launch_bounds__(kI8Threads, 1) hamming_knn2_i8_kernel(const I8
         }
         ++n;
       }
-      if (p.dbg) p.dbg[blockIdx.x * 8 + 3] = (unsigned long long)w_empty;
     }
   } else if (warp == 1) {
     // ===== MMA issuer =====
     if (elect_one()) {
       uint32_t n = 0, g = 0;
       bool probed = false;  // the barrier of the coming tile pair was already seen complete
-      long long w_full = 0;
-      const long long t_start = p.dbg ? clock64() : 0;
       const uint64_t odesc = make_smem_desc(smem_u32(s_ones));
       for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
         const int pair = w / p.q_tiles, qt = w - pair * p.q_tiles;
@@ -416,11 +382,8 @@ __global__ void __launch_bounds__(kI8Threads, 1) hamming_knn2_i8_kernel(const I8
         const uint64_t qdesc = make_smem_desc(smem_u32(s_q + (size_t)qb * kI8TileBytes));
         for (int t = 0; t < n_tt; ++t, ++g) {
           const uint32_t s = g % kI8Stages, a = g & 1u;
-          if (!probed) {  // operands landed AND TMEM stage a drained (first tile pair, item boundaries, late epilogue)
-            const long long c0 = p.dbg ? clock64() : 0;
+          if (!probed)  // operands landed AND TMEM stage a drained (first tile pair, item boundaries, late epilogue)
             mbar_wait_bounded(&b_full[s], (g / kI8Stages) & 1u);
-            if (p.dbg) w_full += clock64() - c0;
-          }
           tc_fence_after();
           const uint64_t tdesc = make_smem_desc(smem_u32(s_t + (size_t)s * kI8TileBytes));
           const uint32_t d1 = tmem_base + a * 256u, d2 = d1 + 128u;
@@ -433,12 +396,6 @@ __global__ void __launch_bounds__(kI8Threads, 1) hamming_knn2_i8_kernel(const I8
         tc_commit(&b_qempty[qb]);  // query tile buffer reusable once this item's MMAs have read it
         ++n;
       }
-      if (p.dbg) {
-        p.dbg[blockIdx.x * 8 + 0] = (unsigned long long)(clock64() - t_start);
-        p.dbg[blockIdx.x * 8 + 1] = 0ull;
-        p.dbg[blockIdx.x * 8 + 2] = (unsigned long long)w_full;
-        p.dbg[blockIdx.x * 8 + 6] = g;
-      }
     }
   } else {
     // ===== epilogue: 2 sets of 4 warps; warp%4 = TMEM lane quarter, set e handles tile pairs with g%2 == e =====
@@ -447,8 +404,6 @@ __global__ void __launch_bounds__(kI8Threads, 1) hamming_knn2_i8_kernel(const I8
     const int row = quarter * 32 + lane;  // TMEM lane = tile row
     const uint32_t lane_addr = tmem_base + ((uint32_t)(quarter * 32) << 16) + eset * 256u;
     uint32_t g = 0;
-    long long w_tfull = 0;
-    const long long e_start = p.dbg ? clock64() : 0;
     for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
       const int pair = w / p.q_tiles, qt = w - pair * p.q_tiles;
       const int qo = p.q_off[pair], nq = p.q_off[pair + 1] - qo;
@@ -463,16 +418,8 @@ __global__ void __launch_bounds__(kI8Threads, 1) hamming_knn2_i8_kernel(const I8
         if ((g & 1u) != eset) continue;
         const int tbase = t * kI8Tile;
         const int nt_valid = min(kI8Tile, nt - tbase);
-        const long long c0 = p.dbg ? clock64() : 0;
         mbar_wait_bounded(&b_tfull[eset], (g >> 1) & 1u);
-        if (p.dbg) w_tfull += clock64() - c0;
         tc_fence_after();
-        if (p.mode & 1) {
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&b_full[(g + 2u) % kI8Stages]);
-          continue;
-        }
         uint32_t v0[32], v1[32], v2[32], v3[32];
         uint32_t b[2] = {kNone, kNone}, s2[2] = {kNone, kNone}, m[2] = {kNone, kNone};
         // D1 columns 0-63 | 64-127, D2 columns 0-63 | 64-127: 128 packed registers, all four
@@ -525,10 +472,6 @@ __global__ void __launch_bounds__(kI8Threads, 1) hamming_knn2_i8_kernel(const I8
       }
       asm volatile("bar.sync 1, 256;" ::: "memory");  // s_merge free for the next item
     }
-    if (p.dbg && threadIdx.x == 64) {
-      p.dbg[blockIdx.x * 8 + 4] = (unsigned long long)(clock64() - e_start);
-      p.dbg[blockIdx.x * 8 + 5] = (unsigned long long)w_tfull;
-    }
   }
 
   tc_fence_before();
@@ -543,26 +486,32 @@ __global__ void __launch_bounds__(kI8Threads, 1) hamming_knn2_i8_kernel(const I8
 // Single-product variant (B2S_VARIANT_I8MMA1): D = Qtile . Ttile^T only.
 //
 // The two-product kernel above spends half of its tensor time on D^T just to make the column
-// minimum a per-thread reduction.  Here the column minimum comes out of D itself: after the
-// index K-step adds the ROW as well as the column (acc = ham*128 + column + row), so the very
-// registers the per-row top-2 was folded from also order a column's entries by (ham, row), and
-// a 5-step butterfly over the 32 lanes of a warp (SUB, IMAD, IMAD, SHFL.BFLY, VIMNMX.U16x2 per
-// surviving register; 62 shuffles) leaves lane L with the minima of columns 4L..4L+3 over the
-// warp's 32 rows.  Each lane widens its four keys and sends them to bwd_best with atomicMin — but only
-// those that beat the current value, which it prefetched before waiting for the accumulator
-// (a stale value merely costs a redundant atomic; ~ln(64) of the 64 candidates per train row
-// and pair survive the filter).
-// Work item = (pair, 256-query block): both 128-row sub-tiles stay in shared memory while
-// the train tiles stream past once, which halves the L2 -> SM operand traffic (at ~650 clk per
-// tile pair 34 KB per tile pair would exceed the L2 slice throughput of the chip).
-// Four TMEM stages of 128 columns (tile pair g uses stage g%4); epilogue set e owns sub-tile e
-// (stages e and e+2), so a thread keeps its row's running top-2 in registers for the whole
-// item and nothing is merged at the end, and the MMA thread runs up to four tile pairs ahead.
+// minimum a per-thread reduction.  Here the column minimum comes out of D itself: the index
+// K-step of the unified tiles adds the ROW as well as the column (see expand_pm8_kernel), so the
+// very registers the per-row top-2 is folded from also order a column's entries by (ham, row).
+// A thread folds the four rows it holds, a 3-level butterfly over the warp leaves lane L with
+// columns 4L..4L+3 over the warp's 32 rows, and the lane widens its four keys and sends them to
+// bwd_best with atomicMin — but only those that beat the current value, which it staged before
+// waiting for the accumulator (a stale value merely costs a redundant atomic; ~ln(64) of the 64
+// candidates per train row and pair survive the filter).
+// Work item = (pair, 256-query block, train part): both 128-row sub-tiles stay in shared memory
+// while the train tiles stream past once, which halves the L2 -> SM operand traffic (at ~650 clk
+// per tile pair 34 KB per tile pair would exceed the L2 slice throughput of the chip).  Four query
+// sub-tiles per item (with a 2-stage ring) halve it again but measured 8 % slower on every
+// BASELINE shape: the epilogue's ALU pipe, not L2, bounds the kernel (DESIGN section 4).
+// Four TMEM stages of 128 columns: tile pair g uses stage g%4 and sub-tile g%2, epilogue set s
+// owns stage s (every other train tile of sub-tile s&1), and the two sets of a sub-tile merge
+// their running top-2 at the end of the item.  The MMA thread runs up to four tile pairs ahead.
 // One barrier per tile pair ("go"): operands landed + TMEM stage drained, probed from inside
 // the MMA stream as above.
 constexpr int kI8sGo = 16;  // go barriers: the producer runs up to 8 tile pairs ahead of the MMA thread
-constexpr int kI8sQTileBytes = (kI8Chunks + 1) * kI8ChunkBytes;  // query tiles carry a zero chunk 17
+constexpr int kI8sQTileBytes = (kI8Chunks + 1) * kI8ChunkBytes;  // unified tiles: 18 chunks
 constexpr int kI8sThreads = 576;  // producer warp + MMA warp + 16 epilogue warps
+constexpr int kI8sSubTiles = 2;   // 128-row query sub-tiles per work item
+constexpr int kI8sStages = 4;     // train-tile ring slots
+constexpr size_t kI8sSmemBytes = (size_t)kI8sSubTiles * kI8sQTileBytes + (size_t)kI8sStages * kI8TileBytes +
+                                 kI8ChunkBytes + 8 * (kI8sGo + 12) + 16 + 4 * kI8Tile * sizeof(uint2) +
+                                 16 * 32 * sizeof(uint4);
 
 __device__ __forceinline__ uint32_t tc_mma_tile_single(uint32_t d, uint64_t qdesc, uint64_t tdesc, uint32_t idesc,
                                                        uint64_t* next_bar, uint32_t next_parity, uint32_t has_next) {
@@ -614,10 +563,10 @@ __device__ __forceinline__ uint32_t tc_mma_tile_single(uint32_t d, uint64_t qdes
 // lower one.  The choice is arithmetic, not SEL: every ALU-pipe instruction (SEL, LOP3, PRMT,
 // VIMNMX) issues at 64 threads/clk/SM on this part (tools/pipe_rates.py) and so does IMAD on
 // the FMA pipe; the epilogue is bound by whichever of the two pipes carries more, so the
-// selection goes to the FMA pipe (3 instructions) and only the minimum stays on the ALU pipe.
+// selection goes to the FMA pipe (3 instructions) and only the maximum stays on the ALU pipe.
 //   e = a - b;  send = up*e + b  (= up ? a : b);  keep = (-up)*e + a  (= up ? b : a)   (exact mod 2^32)
-template <int N, bool MAX = false>
-__device__ __forceinline__ void colmin_step(uint32_t (&y)[64], uint32_t up, uint32_t nup, int lane_mask) {
+template <int N>
+__device__ __forceinline__ void colmin_step(uint32_t (&y)[16], uint32_t up, uint32_t nup, int lane_mask) {
 #pragma unroll
   for (int i = 0; i < N / 2; ++i) {
     uint32_t send, keep;
@@ -633,75 +582,42 @@ __device__ __forceinline__ void colmin_step(uint32_t (&y)[64], uint32_t up, uint
           : "r"(y[i]), "r"(y[i + N / 2]), "r"(up), "r"(nup));
     }
     const uint32_t got = __shfl_xor_sync(0xFFFFFFFFu, send, lane_mask);
-    y[i] = MAX ? __vmaxu2(keep, got) : __vminu2(keep, got);
+    y[i] = __vmaxu2(keep, got);
   }
 }
-
-// Column minima of a 32-row x 128-column slab held one row per lane (64 packed registers).
-// The accumulator already is ham*128 + column + row (see expand_pm8_kernel): within a column
-// (= a register half) the column is the same constant for all lanes, so the unsigned order is
-// the (ham, row) order; rows past the end of the pair arrive as padding keys from the MMA.
-// Five butterfly steps leave lane L with columns 4L..4L+3 in y[0] | y[1]; the column constant
-// is taken off those two registers at the end.
-__device__ __forceinline__ void colmin_warp(uint32_t (&y)[64], int lane) {
-  uint32_t u16 = (lane >> 4) & 1, u8 = (lane >> 3) & 1, u4 = (lane >> 2) & 1, u2 = (lane >> 1) & 1, u1 = lane & 1;
-  colmin_step<64>(y, u16, 0u - u16, 16);
-  colmin_step<32>(y, u8, 0u - u8, 8);
-  colmin_step<16>(y, u4, 0u - u4, 4);
-  colmin_step<8>(y, u2, 0u - u2, 2);
-  colmin_step<4>(y, u1, 0u - u1, 1);
-  const uint32_t cfix = (uint32_t)(4 * lane) * 0x10001u + 0x00010000u;  // columns 4L | 4L+1 of y[0]
-  y[0] -= cfix;
-  y[1] -= cfix + 0x00020002u;                                            // columns 4L+2 | 4L+3
-}
-
-// SUBS = query sub-tiles (128 rows each) that stay in shared memory per work item: 2 (4-stage train ring) or
-// 4 (2-stage ring: a train tile then feeds FOUR tile pairs, ~3400 clk, which still covers the L2 latency of the
-// next one).  With 4 the L2 -> SM operand traffic per tile pair drops from 17 + 2.25 KB to 8.5 + 2.25 KB and
-// epilogue set e simply owns sub-tile e (TMEM stage e), so nothing is merged at the end of an item.
-template <int SUBS> struct I8sCfg {
-  static constexpr int kStages = SUBS == 4 ? 2 : 4;
-  static constexpr size_t kSmem = (size_t)SUBS * kI8sQTileBytes + (size_t)kStages * kI8TileBytes + kI8ChunkBytes +
-                                  8 * (kI8sGo + 12) + 16 + (SUBS == 2 ? 4 * kI8Tile * sizeof(uint2) : 0) +
-                                  16 * 32 * sizeof(uint4);
-};
 
 // TOP2 = false: the per-row SECOND neighbour is not computed (fwd_second stays "none").  The reference's production
 // matcher — BFMatcher(crossCheck=True).match at feature_pipeline.py.bak:82 (cross_check is the default and what
 // configs/pipeline/kitti_default.json sets), persistent_map.py:266, keyframe_manager.py:126,141 — never looks at it;
 // only the kNN + ratio mode (.bak:84-91) and match_orb_descriptors do.  Dropping the second pass removes 64 of the
 // epilogue's ~164 packed min/max instructions per thread and tile pair, and the epilogue's ALU pipe is the kernel's limiter.
-template <int EPI, bool DBG, int SUBS, bool TOP2 = true>
+template <bool TOP2>
 __global__ void __launch_bounds__(kI8sThreads, 1) hamming_knn2_i8s_kernel(const I8Params p) {
-  static_assert(SUBS == 2 || (SUBS == 4 && EPI == 1), "4 sub-tiles per item: 16x256b epilogue only");
-  static_assert(TOP2 || EPI == 1, "best-only: 16x256b epilogue only");
-  constexpr int kStages = I8sCfg<SUBS>::kStages;
   extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* s_q = smem;                                   // SUBS x 36 KB: the item's query sub-tiles (18 chunks each)
-  uint8_t* s_t = smem + SUBS * kI8sQTileBytes;           // kStages x 34 KB
-  uint64_t* bars = reinterpret_cast<uint64_t*>(s_t + kStages * kI8TileBytes + kI8ChunkBytes);  // +1 chunk: see below
+  uint8_t* s_q = smem;                                   // 2 x 36 KB: the item's query sub-tiles (18 chunks each)
+  uint8_t* s_t = smem + kI8sSubTiles * kI8sQTileBytes;   // kI8sStages x 34 KB
+  uint64_t* bars = reinterpret_cast<uint64_t*>(s_t + kI8sStages * kI8TileBytes + kI8ChunkBytes);  // +1 chunk: see below
   uint64_t* b_go = bars;                                 // [kI8sGo]
-  uint64_t* b_empty = bars + kI8sGo;                     // [4] (kStages used)
+  uint64_t* b_empty = bars + kI8sGo;                     // [4] one per ring slot
   uint64_t* b_tfull = bars + kI8sGo + 4;                 // [4] one per TMEM stage
-  uint64_t* b_qempty = bars + kI8sGo + 8;                // [4] (SUBS used)
+  uint64_t* b_qempty = bars + kI8sGo + 8;                // [4] (2 used: one per query sub-tile)
   uint32_t* s_tmem = reinterpret_cast<uint32_t*>(bars + kI8sGo + 12);
-  uint2* s_merge = reinterpret_cast<uint2*>(s_tmem + 4);  // SUBS == 2 only: [2 item parities][2 sub-tiles][128], the two sets of a sub-tile meet here
-  uint4* s_cur = reinterpret_cast<uint4*>(s_merge + (SUBS == 2 ? 4 * kI8Tile : 0));  // [16 epilogue warps][32 lanes]: staged bwd_best values (16x256b epilogue)
+  uint2* s_merge = reinterpret_cast<uint2*>(s_tmem + 4);  // [2 item parities][2 sub-tiles][128], the two sets of a sub-tile meet here
+  uint4* s_cur = reinterpret_cast<uint4*>(s_merge + 4 * kI8Tile);  // [16 epilogue warps][32 lanes]: staged bwd_best values
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int q_blocks = (p.q_tiles + SUBS - 1) / SUBS;
+  const int q_blocks = (p.q_tiles + kI8sSubTiles - 1) / kI8sSubTiles;
   const int t_split = p.t_split;
   const int n_items = p.n_pairs * q_blocks * t_split;    // item w = ((pair * q_blocks) + qb) * t_split + part
 
   // the index K-step reads one chunk past the last ring slot (times the query tile's zero chunk):
-  // keep that chunk inside the allocation and defined
+  // keep that chunk inside the allocation and defined; the query slots' chunk 17 is never loaded
+  // and must read as zero
   for (int i = threadIdx.x; i < kI8Tile; i += kI8sThreads) {
-    reinterpret_cast<uint4*>(s_t + kStages * kI8TileBytes)[i] = make_uint4(0u, 0u, 0u, 0u);
-    if (EPI == 1) {  // unified tiles: the query slots' chunk 17 is never loaded and must read as zero
+    reinterpret_cast<uint4*>(s_t + kI8sStages * kI8TileBytes)[i] = make_uint4(0u, 0u, 0u, 0u);
 #pragma unroll
-      for (int sub = 0; sub < SUBS; ++sub)
-        reinterpret_cast<uint4*>(s_q + sub * kI8sQTileBytes + kI8TileBytes)[i] = make_uint4(0u, 0u, 0u, 0u);
-    }
+    for (int sub = 0; sub < kI8sSubTiles; ++sub)
+      reinterpret_cast<uint4*>(s_q + sub * kI8sQTileBytes + kI8TileBytes)[i] = make_uint4(0u, 0u, 0u, 0u);
   }
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
 
@@ -724,8 +640,8 @@ __global__ void __launch_bounds__(kI8sThreads, 1) hamming_knn2_i8s_kernel(const 
   tc_fence_after();
   const uint32_t tmem_base = *s_tmem;
 
-  // all roles walk the same items; an item always has SUBS * (t1 - t0) tile pairs (trailing sub-tiles may
-  // be all padding: their MMAs then read stale shared memory and every result is ignored)
+  // all roles walk the same items; an item always has 2 (t1 - t0) tile pairs (a trailing sub-tile may
+  // be all padding: its MMAs then read stale shared memory and every result is ignored)
 #define B2S_I8S_ITEM(w)                                                                          \
   const int part = (w) % t_split, pq = (w) / t_split;                                            \
   const int pair = pq / q_blocks, qb = pq - pair * q_blocks;                                     \
@@ -733,261 +649,113 @@ __global__ void __launch_bounds__(kI8sThreads, 1) hamming_knn2_i8s_kernel(const 
   const int to = p.t_off[pair], nt = p.t_off[pair + 1] - to;                                     \
   const int n_tt = (nt + kI8Tile - 1) / kI8Tile;                                                 \
   const int t0 = (int)(((long long)part * n_tt) / t_split), t1 = (int)(((long long)(part + 1) * n_tt) / t_split); \
-  if (qb * SUBS * kI8Tile >= nq || t0 >= t1) continue;
+  if (qb * kI8sSubTiles * kI8Tile >= nq || t0 >= t1) continue;
   if (warp == 0) {
     // ===== producer =====
     if (lane == 0) {
       uint32_t n = 0, tau = 0;  // items / train tiles seen by this CTA
-      long long w_empty = 0;
       for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
         B2S_I8S_ITEM(w)
         (void)to;
-        const int q0 = qb * SUBS * kI8Tile;
-        // EPI 1: unified 18-chunk tiles on both sides; a train slot takes chunks 0..16 (data + its B-side
-        // index chunk, one copy), a query slot chunks 0..15 and chunk 17 (its A-side index chunk, two copies
+        const int q0 = qb * kI8sSubTiles * kI8Tile;
+        // unified 18-chunk tiles on both sides: a train slot takes chunks 0..16 (data + its B-side index
+        // chunk, one copy), a query slot chunks 0..15 and chunk 17 (its A-side index chunk, two copies
         // once per item)
-        constexpr uint32_t kTStride = EPI == 1 ? (uint32_t)kI8sQTileBytes : (uint32_t)kI8TileBytes;
-        constexpr uint32_t kQBytes = EPI == 1 ? (uint32_t)kI8TileBytes : (uint32_t)kI8sQTileBytes;
         const size_t t_tile0 = p.t_xt ? (size_t)p.t_xt[pair] : (size_t)pair * p.t_tiles;
         const size_t q_tile0 = p.q_xt ? (size_t)p.q_xt[pair] : (size_t)pair * p.q_tiles;
-        const uint8_t* tsrc = p.tx + t_tile0 * kTStride;
-        const uint8_t* qsrc = p.qx + (q_tile0 + (size_t)SUBS * qb) * kI8sQTileBytes;
+        const uint8_t* tsrc = p.tx + t_tile0 * kI8sQTileBytes;
+        const uint8_t* qsrc = p.qx + (q_tile0 + (size_t)kI8sSubTiles * qb) * kI8sQTileBytes;
         for (int t = t0; t < t1; ++t, ++tau) {
-          const uint32_t s = tau % kStages, g = (uint32_t)SUBS * tau;
-          const long long c0 = p.dbg ? clock64() : 0;
-          if (tau >= (uint32_t)kStages) mbar_wait_bounded(&b_empty[s], ((tau / kStages) - 1u) & 1u);
-          if (p.dbg) w_empty += clock64() - c0;
-          const bool skip_t = (p.mode & 2) && tau >= (uint32_t)kStages;
+          const uint32_t s = tau % kI8sStages, g = (uint32_t)kI8sSubTiles * tau;
+          if (tau >= (uint32_t)kI8sStages) mbar_wait_bounded(&b_empty[s], ((tau / kI8sStages) - 1u) & 1u);
 #pragma unroll
-          for (int sub = 0; sub < SUBS; ++sub) {
+          for (int sub = 0; sub < kI8sSubTiles; ++sub) {
             uint64_t* go = &b_go[(g + (uint32_t)sub) % kI8sGo];
             const bool load_q = t == t0 && q0 + sub * kI8Tile < nq;   // the item's query sub-tile rides on its first tile pair
-            const uint32_t t_bytes = (sub == 0 && !skip_t) ? (uint32_t)kI8TileBytes : 0u;
+            const uint32_t t_bytes = sub == 0 ? (uint32_t)kI8TileBytes : 0u;   // the train tile rides on sub-tile 0
             if (load_q) {
               if (n >= 1) mbar_wait_bounded(&b_qempty[sub], (n - 1u) & 1u);
-              mbar_arrive_expect_tx(go, kQBytes + t_bytes);
+              mbar_arrive_expect_tx(go, (uint32_t)kI8TileBytes + t_bytes);
               uint8_t* qdst = s_q + sub * kI8sQTileBytes;
               const uint8_t* qs = qsrc + (size_t)sub * kI8sQTileBytes;
-              if (EPI == 1) {
-                bulk_g2s(qdst, qs, 16 * kI8ChunkBytes, go);
-                bulk_g2s(qdst + 16 * kI8ChunkBytes, qs + 17 * kI8ChunkBytes, kI8ChunkBytes, go);
-              } else {
-                bulk_g2s(qdst, qs, kQBytes, go);
-              }
+              bulk_g2s(qdst, qs, 16 * kI8ChunkBytes, go);
+              bulk_g2s(qdst + 16 * kI8ChunkBytes, qs + 17 * kI8ChunkBytes, kI8ChunkBytes, go);
             } else if (t_bytes) {
               mbar_arrive_expect_tx(go, t_bytes);
             } else {
               mbar_arrive(go);
             }
-            if (t_bytes) bulk_g2s(s_t + (size_t)s * kI8TileBytes, tsrc + (size_t)t * kTStride, kI8TileBytes, go);
+            if (t_bytes) bulk_g2s(s_t + (size_t)s * kI8TileBytes, tsrc + (size_t)t * kI8sQTileBytes, kI8TileBytes, go);
           }
         }
         ++n;
       }
-      if (p.dbg) p.dbg[blockIdx.x * 8 + 3] = (unsigned long long)w_empty;
     }
   } else if (warp == 1) {
     // ===== MMA issuer =====
     if (elect_one()) {
       uint32_t g = 0;
       bool probed = false;
-      long long w_full = 0;
-      const long long t_start = p.dbg ? clock64() : 0;
-      uint64_t qdesc[SUBS];
+      uint64_t qdesc[kI8sSubTiles];
 #pragma unroll
-      for (int sub = 0; sub < SUBS; ++sub) qdesc[sub] = make_smem_desc(smem_u32(s_q + sub * kI8sQTileBytes));
+      for (int sub = 0; sub < kI8sSubTiles; ++sub) qdesc[sub] = make_smem_desc(smem_u32(s_q + sub * kI8sQTileBytes));
       for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
         B2S_I8S_ITEM(w)
         (void)to;
         for (int t = t0; t < t1; ++t) {
-          const uint32_t s = (g / (uint32_t)SUBS) % kStages;
+          const uint32_t s = (g / (uint32_t)kI8sSubTiles) % kI8sStages;
           const uint64_t tdesc = make_smem_desc(smem_u32(s_t + (size_t)s * kI8TileBytes));
 #pragma unroll
-          for (uint32_t sub = 0; sub < (uint32_t)SUBS; ++sub, ++g) {
-            if (!probed) {  // first tile pair, item boundaries, late epilogue or late loads
-              const long long c0 = p.dbg ? clock64() : 0;
+          for (uint32_t sub = 0; sub < (uint32_t)kI8sSubTiles; ++sub, ++g) {
+            if (!probed)  // first tile pair, item boundaries, late epilogue or late loads
               mbar_wait_bounded(&b_go[g % kI8sGo], (g / kI8sGo) & 1u);
-              if (p.dbg) w_full += clock64() - c0;
-            }
             tc_fence_after();
             const uint32_t gn = g + 1u;
-            const uint32_t more = (sub + 1u < (uint32_t)SUBS || t + 1 < t1) ? 1u : 0u;
+            const uint32_t more = (sub + 1u < (uint32_t)kI8sSubTiles || t + 1 < t1) ? 1u : 0u;
             probed = tc_mma_tile_single(tmem_base + (g & 3u) * 128u, qdesc[sub], tdesc, kIdescI8,
                                         &b_go[gn % kI8sGo], (gn / kI8sGo) & 1u, more) != 0u;
-            if (sub == (uint32_t)SUBS - 1u) tc_commit(&b_empty[s]);  // train tile consumed by every sub-tile
+            if (sub == (uint32_t)kI8sSubTiles - 1u) tc_commit(&b_empty[s]);  // train tile consumed by every sub-tile
             tc_commit(&b_tfull[g & 3u]);                    // accumulator stage complete
             if (t == t1 - 1) tc_commit(&b_qempty[sub]);     // the item's last use of this query sub-tile
           }
         }
       }
-      if (p.dbg) {
-        p.dbg[blockIdx.x * 8 + 0] = (unsigned long long)(clock64() - t_start);
-        p.dbg[blockIdx.x * 8 + 1] = 0ull;
-        p.dbg[blockIdx.x * 8 + 2] = (unsigned long long)w_full;
-        p.dbg[blockIdx.x * 8 + 6] = g;
-      }
     }
   } else {
-    if constexpr (EPI == 0) {
     // ===== epilogue: 4 sets of 4 warps; set s owns TMEM stage s, i.e. the tile pairs g with g%4 == s
     // (sub-tile s&1, every other train tile); warp%4 = TMEM lane quarter.  Four warps per scheduler
     // instead of two: the per-tile-pair work is a long dependent chain (TMEM load, folds, butterfly)
-    // and two warps left the ALU and FMA pipes half idle. =====
-    const int quarter = warp & 3;
-    const uint32_t set = (uint32_t)(warp - 2) >> 2;
-    const uint32_t sub = set & 1u;
-    const int row = quarter * 32 + lane;  // TMEM lane = row of the sub-tile
-    const uint32_t lane_addr = tmem_base + ((uint32_t)(quarter * 32) << 16) + set * 128u;
-    uint32_t g_item = 0, hs = 0, n = 0;  // first tile pair of the item, tile pairs handled by this set, items
-    long long w_tfull = 0;
-    const long long e_start = p.dbg ? clock64() : 0;
-    for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
-      B2S_I8S_ITEM(w)
-      const int qo = p.q_off[pair];
-      const int q0 = qb * 2 * kI8Tile + (int)sub * kI8Tile;   // first query row of this set's sub-tile
-      const int rows_valid = max(0, min(kI8Tile, nq - q0));
-      uint32_t gbest = kNone, gsecond = kNone;
-      for (int t = t0; t < t1; ++t) {
-        const uint32_t g = g_item + 2u * (uint32_t)(t - t0) + sub;
-        if ((g & 3u) != set) continue;
-        const int tbase = t * kI8Tile;
-        const int nt_valid = min(kI8Tile, nt - tbase);
-        // current column minima of this lane's 4 train rows (stale is fine: only used to skip atomics)
-        uint32_t cur[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          const int c = 4 * lane + k;
-          cur[k] = (c < nt_valid) ? __ldcg(&p.bwd_best[to + tbase + c]) : 0u;
-        }
-        const long long c0 = p.dbg ? clock64() : 0;
-        mbar_wait_bounded(&b_tfull[set], hs & 1u);
-        ++hs;
-        if (p.dbg) w_tfull += clock64() - c0;
-        tc_fence_after();
-        if (p.mode & 1) {
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&b_go[(g + 4u) % kI8sGo]);
-          continue;
-        }
-        uint32_t y[64];
-        {
-          uint32_t v0[32], v1[32];
-          TMEM_LD_X32P(lane_addr, v0);
-          TMEM_LD_X32P(lane_addr + 64u, v1);
-          tmem_ld_wait();
-          TMEM_REGS_READY(v0);
-          TMEM_REGS_READY(v1);
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            y[j] = v0[j];
-            y[j + 32] = v1[j];
-          }
-        }
-        tc_fence_before();
-        __syncwarp();
-        // accumulator drained into registers: the stage goes to tile pair g+4 (same sub-tile, two train tiles on)
-        if (lane == 0) mbar_arrive(&b_go[(g + 4u) % kI8sGo]);
-        // ---- per-row top-2 of this tile, two passes over the 64 packed registers ----
-        // pass 1: minimum per 16-bit lane (even / odd columns), VIMNMX3: 0.5 instruction per register.
-        // pass 2: keys are unique within a row (the column is part of the key), so with c = ~best
-        // (= -(best + 1) per half-word) the wrapped sum x + c is 0xFFFF exactly for the minimum itself
-        // and x - best - 1 (order preserving) for everything else; VIADDMNMX.U16x2 adds and takes
-        // the running minimum in ONE instruction per register.  1.5 per register instead of 2.5.
-        if (!(p.mode & 8)) {
-          uint32_t m[2] = {kNone, kNone}, a2[2] = {kNone, kNone};
-#pragma unroll
-          for (int j = 0; j < 64; j += 4) {
-            m[0] = __vimin3_u16x2(m[0], y[j], y[j + 1]);
-            m[1] = __vimin3_u16x2(m[1], y[j + 2], y[j + 3]);
-          }
-          const uint32_t bb = __vminu2(m[0], m[1]);
-          const uint32_t cneg = ~bb;
-#pragma unroll
-          for (int j = 0; j < 64; j += 2) {
-            a2[0] = __viaddmin_u16x2(y[j], cneg, a2[0]);
-            a2[1] = __viaddmin_u16x2(y[j + 1], cneg, a2[1]);
-          }
-          const uint32_t ss = __vminu2(a2[0], a2[1]) + bb + 0x00010001u;  // second per 16-bit lane (no carry: < 2^16 each)
-          const uint32_t bw = swap16(bb);
-          const uint32_t best16 = __vminu2(bb, bw);
-          const uint32_t sec16 = __vimin3_u16x2(__vmaxu2(bb, bw), ss, swap16(ss));
-          // keys carry + row (constant per thread): take it off before widening
-          top2_insert(gbest, gsecond, key16_to_key32((best16 & 0xFFFFu) - (uint32_t)row, (uint32_t)tbase));
-          top2_insert(gbest, gsecond, key16_to_key32((sec16 & 0xFFFFu) - (uint32_t)row, (uint32_t)tbase));
-        }
-        // ---- column minima: butterfly over the warp on the very same registers ----
-        if (!(p.mode & 4)) colmin_warp(y, lane);
-        // lane L now holds columns 4L..4L+3 (y[0] = 4L | 4L+1, y[1] = 4L+2 | 4L+3) over this warp's 32 rows;
-        // a candidate that does not beat the (possibly stale) current minimum needs no atomic
-        const uint32_t cm16[4] = {y[0] & 0xFFFFu, y[0] >> 16, y[1] & 0xFFFFu, y[1] >> 16};
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          const uint32_t key = key16_to_key32(cm16[k], (uint32_t)q0);
-          // rows_valid == 0: the whole sub-tile is padding and its MMAs read stale shared memory
-          if (rows_valid > 0 && cm16[k] < kKey16Valid && key < cur[k]) atomicMin(&p.bwd_best[to + tbase + 4 * lane + k], key);
-        }
-      }
-      g_item += 2u * (uint32_t)(t1 - t0);
-      // the two sets of a sub-tile (even / odd train tiles) meet in shared memory; double buffered by
-      // item parity, so one named barrier per item is enough
-      uint2* mg = s_merge + (((n & 1u) * 2u + sub) << 7);
-      if (set >= 2u) mg[row] = make_uint2(gbest, gsecond);
-      asm volatile("bar.sync %0, 256;" ::"r"(1u + sub) : "memory");  // the 8 warps of this sub-tile
-      if (set < 2u && row < rows_valid) {
-        const uint2 o = mg[row];
-        top2_insert(gbest, gsecond, o.x);
-        top2_insert(gbest, gsecond, o.y);
-        const uint32_t ob = gbest >= kKey32Pad ? kNone : gbest, os = gsecond >= kKey32Pad ? kNone : gsecond;
-        if (t_split > 1) {
-          p.partial[(size_t)part * p.total_nq + qo + q0 + row] = make_uint2(ob, os);
-        } else {
-          p.fwd_best[qo + q0 + row] = ob;
-          p.fwd_second[qo + q0 + row] = os;
-        }
-      }
-      ++n;
-    }
-    if (p.dbg && threadIdx.x == 64) {
-      p.dbg[blockIdx.x * 8 + 4] = (unsigned long long)(clock64() - e_start);
-      p.dbg[blockIdx.x * 8 + 5] = (unsigned long long)w_tfull;
-    }
-    } else {
-    // ===== epilogue, 16x256b form (default): same sets / stages / barriers as above, but the accumulator
-    // is read with tcgen05.ld.16x256b: a thread then owns 4 ROWS (gr, gr+8, gr+16, gr+24 of its warp's
-    // 32 TMEM lanes, gr = lane/4) x 32 columns (eight 4-column groups, 16 g + 4 (lane%4) ..+3) instead
-    // of 1 row x 128 columns.
+    // and two warps left the ALU and FMA pipes half idle.  The accumulator is read with
+    // tcgen05.ld.16x256b: a thread owns 4 ROWS (gr, gr+8, gr+16, gr+24 of its warp's 32 TMEM lanes,
+    // gr = lane/4) x 32 columns (eight 4-column groups, 16 g + 4 (lane%4) ..+3).
     //  * Column minimum: the four rows are folded inside the thread (2 instructions per register) and
-    //    only then cross lanes: 3 butterfly levels over 16 registers (14 exchanges) instead of 5 levels
-    //    over 64 (62 exchanges); it ends with lane L holding columns 4L..4L+3 exactly as before.
+    //    only then cross lanes: 3 butterfly levels over 16 registers (14 exchanges) leave lane L holding
+    //    columns 4L..4L+3.
     //  * Per-row top-2: 16 registers per row, two rows in lock step (independent dependency chains: with
     //    64 of the 96 registers holding the accumulator ptxas otherwise runs one serial chain at a time
     //    and the epilogue is latency-, not issue-bound); the results of two rows share a register
     //    (row a | row b << 16), the four lanes that share a row merge in that packed form (4 SHFL per
-    //    level) and lane%4 = k finishes row k: one running top-2 per thread, as in the 32x32b form. =====
+    //    level) and lane%4 = k finishes row k: one running top-2 per thread. =====
     const int quarter = warp & 3;
     const uint32_t set = (uint32_t)(warp - 2) >> 2;
-    const uint32_t sub = SUBS == 4 ? set : (set & 1u);
+    const uint32_t sub = set & 1u;
     const int gr = lane >> 2, tc = lane & 3;
     const int row = quarter * 32 + gr + 8 * tc;   // the tile-local row this lane keeps the running top-2 of
     const uint32_t row_base = (uint32_t)(quarter * 32 + gr);
     const uint32_t pick = tc == 0 ? 0x3210u : tc == 1 ? 0x1032u : tc == 2 ? 0x7654u : 0x5476u;  // row k = tc -> low half
     const uint32_t lane_addr = tmem_base + ((uint32_t)(quarter * 32) << 16) + set * 128u;
-    uint32_t g_item = 0, hs = 0, n = 0;
-    long long w_tfull = 0;
-    const long long e_start = DBG ? clock64() : 0;
+    uint32_t g_item = 0, n = 0;  // first tile pair of the item, items
     for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
       B2S_I8S_ITEM(w)
-      const int q0 = qb * SUBS * kI8Tile + (int)sub * kI8Tile;
+      const int q0 = qb * kI8sSubTiles * kI8Tile + (int)sub * kI8Tile;   // first query row of this set's sub-tile
       const int rows_valid = max(0, min(kI8Tile, nq - q0));
       const bool staged = (reinterpret_cast<uintptr_t>(p.bwd_best + to) & 15u) == 0;   // cp.async.cg moves 16 aligned bytes
       uint32_t gbest = kNone, gsecond = kNone;
-      // this set's tile pairs: g = g_item + SUBS k + sub (k = t - t0) with g % 4 == set: every train tile of
-      // sub-tile `set` (SUBS == 4), every other train tile of sub-tile set & 1 (SUBS == 2)
-      constexpr int kStep = SUBS == 4 ? 1 : 2;
-      for (int k = SUBS == 4 ? 0 : (int)(((set >> 1) ^ (g_item >> 1)) & 1u); k < t1 - t0; k += kStep) {
-        const int t = t0 + k;
-        const uint32_t g = g_item + (uint32_t)SUBS * (uint32_t)k + sub;
+      // this set's tile pairs: g = g_item + 2 (t - t0) + sub with g % 4 == set, i.e. every other train tile;
+      // stage `set` has served g / 4 tile pairs before g
+      const uint32_t g_end = g_item + (uint32_t)kI8sSubTiles * (uint32_t)(t1 - t0);
+      for (uint32_t g = (g_item + 3u - set) / 4u * 4u + set; g < g_end; g += 4u) {
+        const int t = t0 + (int)((g - g_item) >> 1);
         const int tbase = t * kI8Tile;
         // current column minima of this lane's 4 train rows (stale is fine: only used to skip atomics).
         // Holding them in registers through the top-2 costs more than it saves (96 registers, 64 of them
@@ -1003,17 +771,8 @@ __global__ void __launch_bounds__(kI8sThreads, 1) hamming_knn2_i8s_kernel(const 
           asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n\tcp.async.commit_group;"
                        ::"r"(smem_u32(cur_slot)), "l"(src), "r"(nbytes) : "memory");
         }
-        const long long c0 = DBG ? clock64() : 0;
-        mbar_wait_bounded(&b_tfull[set], hs & 1u);
-        ++hs;
-        if (DBG) w_tfull += clock64() - c0;
+        mbar_wait_bounded(&b_tfull[set], (g >> 2) & 1u);
         tc_fence_after();
-        if (p.mode & 1) {
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&b_go[(g + 4u) % kI8sGo]);
-          continue;
-        }
         uint32_t ra[32], rb[32];
         TMEM_LD_16X256_X8P(lane_addr, ra);
         TMEM_LD_16X256_X8P(lane_addr + (16u << 16), rb);
@@ -1028,94 +787,88 @@ __global__ void __launch_bounds__(kI8sThreads, 1) hamming_knn2_i8s_kernel(const 
 #define B2S_R1(r, i) (r[4 * ((i) >> 1) + 2 + ((i) & 1)])
         // ---- per-row top-2 of this tile: rows (0, 1) from ra, rows (2, 3) from rb, two rows in lock step ----
         uint32_t pb[2], ps[2];  // packed results: row a in the low half, row b in the high half
-        if (!(p.mode & 8)) {
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          const uint32_t(&r)[32] = h ? rb : ra;
+          // pass 1: minimum per 16-bit lane (even / odd columns of the 4-column groups)
+          uint32_t m0 = __vimax3_u16x2(B2S_R0(r, 0), B2S_R0(r, 1), B2S_R0(r, 2));
+          uint32_t m1 = __vimax3_u16x2(B2S_R1(r, 0), B2S_R1(r, 1), B2S_R1(r, 2));
+#pragma unroll
+          for (int i = 3; i < 15; i += 2) {
+            m0 = __vimax3_u16x2(m0, B2S_R0(r, i), B2S_R0(r, i + 1));
+            m1 = __vimax3_u16x2(m1, B2S_R1(r, i), B2S_R1(r, i + 1));
+          }
+          const uint32_t bb0 = __vmaxu2(m0, B2S_R0(r, 15)), bb1 = __vmaxu2(m1, B2S_R1(r, 15));
+          // fold the even / odd halves of both rows at once: x = (row a even | row b even), y = (.. odd | .. odd)
+          const uint32_t x = __byte_perm(bb0, bb1, 0x5410), y = __byte_perm(bb0, bb1, 0x7632);
+          pb[h] = __vmaxu2(x, y);
+          if constexpr (TOP2) {
+            // pass 2: values are unique within a row (or zero padding, never the largest of a real row), so
+            // x - best wraps to 0 exactly for the maximum itself and keeps the order of everything below it
+            const uint32_t cn0 = __vneg2(bb0), cn1 = __vneg2(bb1);
+            uint32_t a00 = 0u, a01 = 0u, a10 = 0u, a11 = 0u;
+#pragma unroll
+            for (int i = 0; i < 16; i += 2) {
+              a00 = __viaddmax_u16x2(B2S_R0(r, i), cn0, a00);
+              a10 = __viaddmax_u16x2(B2S_R1(r, i), cn1, a10);
+              a01 = __viaddmax_u16x2(B2S_R0(r, i + 1), cn0, a01);
+              a11 = __viaddmax_u16x2(B2S_R1(r, i + 1), cn1, a11);
+            }
+            const uint32_t ss0 = __vadd2(__vmaxu2(a00, a01), bb0);  // second largest per 16-bit lane (mod 2^16 per lane)
+            const uint32_t ss1 = __vadd2(__vmaxu2(a10, a11), bb1);
+            const uint32_t sx = __byte_perm(ss0, ss1, 0x5410), sy = __byte_perm(ss0, ss1, 0x7632);
+            ps[h] = __vimax3_u16x2(__vminu2(x, y), sx, sy);
+          }
+        }
+        // the four lanes that share these rows hold disjoint columns: merge best / second, both row pairs
+#pragma unroll
+        for (int o = 1; o <= 2; o <<= 1) {
 #pragma unroll
           for (int h = 0; h < 2; ++h) {
-            const uint32_t(&r)[32] = h ? rb : ra;
-            // pass 1: minimum per 16-bit lane (even / odd columns of the 4-column groups)
-            uint32_t m0 = __vimax3_u16x2(B2S_R0(r, 0), B2S_R0(r, 1), B2S_R0(r, 2));
-            uint32_t m1 = __vimax3_u16x2(B2S_R1(r, 0), B2S_R1(r, 1), B2S_R1(r, 2));
-#pragma unroll
-            for (int i = 3; i < 15; i += 2) {
-              m0 = __vimax3_u16x2(m0, B2S_R0(r, i), B2S_R0(r, i + 1));
-              m1 = __vimax3_u16x2(m1, B2S_R1(r, i), B2S_R1(r, i + 1));
-            }
-            const uint32_t bb0 = __vmaxu2(m0, B2S_R0(r, 15)), bb1 = __vmaxu2(m1, B2S_R1(r, 15));
-            // fold the even / odd halves of both rows at once: x = (row a even | row b even), y = (.. odd | .. odd)
-            const uint32_t x = __byte_perm(bb0, bb1, 0x5410), y = __byte_perm(bb0, bb1, 0x7632);
-            pb[h] = __vmaxu2(x, y);
+            const uint32_t ob = __shfl_xor_sync(0xFFFFFFFFu, pb[h], o);
             if constexpr (TOP2) {
-              // pass 2: values are unique within a row (or zero padding, never the largest of a real row), so
-              // x - best wraps to 0 exactly for the maximum itself and keeps the order of everything below it
-              const uint32_t cn0 = __vneg2(bb0), cn1 = __vneg2(bb1);
-              uint32_t a00 = 0u, a01 = 0u, a10 = 0u, a11 = 0u;
-#pragma unroll
-              for (int i = 0; i < 16; i += 2) {
-                a00 = __viaddmax_u16x2(B2S_R0(r, i), cn0, a00);
-                a10 = __viaddmax_u16x2(B2S_R1(r, i), cn1, a10);
-                a01 = __viaddmax_u16x2(B2S_R0(r, i + 1), cn0, a01);
-                a11 = __viaddmax_u16x2(B2S_R1(r, i + 1), cn1, a11);
-              }
-              const uint32_t ss0 = __vadd2(__vmaxu2(a00, a01), bb0);  // second largest per 16-bit lane (mod 2^16 per lane)
-              const uint32_t ss1 = __vadd2(__vmaxu2(a10, a11), bb1);
-              const uint32_t sx = __byte_perm(ss0, ss1, 0x5410), sy = __byte_perm(ss0, ss1, 0x7632);
-              ps[h] = __vimax3_u16x2(__vminu2(x, y), sx, sy);
+              const uint32_t os = __shfl_xor_sync(0xFFFFFFFFu, ps[h], o);
+              ps[h] = __vimax3_u16x2(__vminu2(pb[h], ob), ps[h], os);
             }
+            pb[h] = __vmaxu2(pb[h], ob);
           }
-          // the four lanes that share these rows hold disjoint columns: merge best / second, both row pairs
-#pragma unroll
-          for (int o = 1; o <= 2; o <<= 1) {
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {
-              const uint32_t ob = __shfl_xor_sync(0xFFFFFFFFu, pb[h], o);
-              if constexpr (TOP2) {
-                const uint32_t os = __shfl_xor_sync(0xFFFFFFFFu, ps[h], o);
-                ps[h] = __vimax3_u16x2(__vminu2(pb[h], ob), ps[h], os);
-              }
-              pb[h] = __vmaxu2(pb[h], ob);
-            }
-          }
-          // lane%4 = k finishes row k: complement (acc = ~key), then the keys carry + row: take it off before widening
-          const uint32_t best16 = ~__byte_perm(pb[0], pb[1], pick) & 0xFFFFu;
-          if constexpr (TOP2) {
-            const uint32_t sec16 = ~__byte_perm(ps[0], ps[1], pick) & 0xFFFFu;
-            top2_insert(gbest, gsecond, key16_to_key32(best16 - (uint32_t)row, (uint32_t)tbase));
-            top2_insert(gbest, gsecond, key16_to_key32(sec16 - (uint32_t)row, (uint32_t)tbase));
-          } else {
-            gbest = min(gbest, key16_to_key32(best16 - (uint32_t)row, (uint32_t)tbase));
-          }
+        }
+        // lane%4 = k finishes row k: complement (acc = ~key), then the keys carry + row: take it off before widening
+        const uint32_t best16 = ~__byte_perm(pb[0], pb[1], pick) & 0xFFFFu;
+        if constexpr (TOP2) {
+          const uint32_t sec16 = ~__byte_perm(ps[0], ps[1], pick) & 0xFFFFu;
+          top2_insert(gbest, gsecond, key16_to_key32(best16 - (uint32_t)row, (uint32_t)tbase));
+          top2_insert(gbest, gsecond, key16_to_key32(sec16 - (uint32_t)row, (uint32_t)tbase));
+        } else {
+          gbest = min(gbest, key16_to_key32(best16 - (uint32_t)row, (uint32_t)tbase));
         }
         // ---- column minima: the 4 rows inside the thread, then 3 butterfly levels over lane bits 2..4 ----
-        uint32_t y[64];   // colmin_step's signature; only y[0..15] are live
+        uint32_t y[16];
         uint32_t cur[4] = {0u, 0u, 0u, 0u};
-        if (!(p.mode & 4)) {
 #pragma unroll
-          for (int i = 0; i < 16; ++i) y[i] = __vmaxu2(__vimax3_u16x2(B2S_R0(ra, i), B2S_R1(ra, i), B2S_R0(rb, i)), B2S_R1(rb, i));
-          // current column minima of this lane's 4 train rows (stale is fine: only used to skip atomics):
-          // requested here, into the accumulator registers the fold just freed, and consumed after the
-          // butterfly (requesting them before the accumulator wait costs 4 registers through the top-2
-          // and measured slower: 892 vs 876 clk per tile pair)
-          if (!staged) {
-            const int nt_valid = min(kI8Tile, nt - tbase);
+        for (int i = 0; i < 16; ++i) y[i] = __vmaxu2(__vimax3_u16x2(B2S_R0(ra, i), B2S_R1(ra, i), B2S_R0(rb, i)), B2S_R1(rb, i));
+        // current column minima of this lane's 4 train rows (stale is fine: only used to skip atomics):
+        // requested here, into the accumulator registers the fold just freed, and consumed after the
+        // butterfly (requesting them before the accumulator wait costs 4 registers through the top-2
+        // and measured slower: 892 vs 876 clk per tile pair)
+        if (!staged) {
+          const int nt_valid = min(kI8Tile, nt - tbase);
 #pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const int c = 4 * lane + k;
-              cur[k] = (c < nt_valid) ? __ldcg(&p.bwd_best[to + tbase + c]) : 0u;
-            }
+          for (int k = 0; k < 4; ++k) {
+            const int c = 4 * lane + k;
+            cur[k] = (c < nt_valid) ? __ldcg(&p.bwd_best[to + tbase + c]) : 0u;
           }
-          const uint32_t u16 = (lane >> 4) & 1, u8 = (lane >> 3) & 1, u4 = (lane >> 2) & 1;
-          colmin_step<16, true>(y, u16, 0u - u16, 16);
-          colmin_step<8, true>(y, u8, 0u - u8, 8);
-          colmin_step<4, true>(y, u4, 0u - u4, 4);
-          // register i of lane L is now position 2 (L/4) + i, i.e. columns 16 (L/4) + 4 (L%4) + 2 i, +1 = 4 L + 2 i, +1
-          // acc = 65535 - (128 ham + column + row): complement and take the column off in one subtraction
-          // (no borrow between the halves: 65535 - column >= acc)
-          const uint32_t cfix = (uint32_t)(4 * lane) * 0x10001u + 0x00010000u;
-          y[0] = (0xFFFFFFFFu - cfix) - y[0];
-          y[1] = (0xFFFFFFFFu - cfix - 0x00020002u) - y[1];
-        } else {
-          y[0] = y[1] = kNone;
         }
+        const uint32_t u16 = (lane >> 4) & 1, u8 = (lane >> 3) & 1, u4 = (lane >> 2) & 1;
+        colmin_step<16>(y, u16, 0u - u16, 16);
+        colmin_step<8>(y, u8, 0u - u8, 8);
+        colmin_step<4>(y, u4, 0u - u4, 4);
+        // register i of lane L is now position 2 (L/4) + i, i.e. columns 16 (L/4) + 4 (L%4) + 2 i, +1 = 4 L + 2 i, +1
+        // acc = 65535 - (128 ham + column + row): complement and take the column off in one subtraction
+        // (no borrow between the halves: 65535 - column >= acc)
+        const uint32_t cfix = (uint32_t)(4 * lane) * 0x10001u + 0x00010000u;
+        y[0] = (0xFFFFFFFFu - cfix) - y[0];
+        y[1] = (0xFFFFFFFFu - cfix - 0x00020002u) - y[1];
         if (staged) {
           asm volatile("cp.async.wait_group 0;" ::: "memory");
           const uint4 c4 = *cur_slot;
@@ -1131,22 +884,16 @@ __global__ void __launch_bounds__(kI8sThreads, 1) hamming_knn2_i8s_kernel(const 
           if (rows_valid > 0 && cm16[k] < kKey16Valid && key < cur[k]) atomicMin(&p.bwd_best[to + tbase + 4 * lane + k], key);
         }
       }
-      g_item += (uint32_t)SUBS * (uint32_t)(t1 - t0);
-      bool writer = row < rows_valid;
-      if (SUBS == 2) {
-        // the two sets of a sub-tile (even / odd train tiles) meet in shared memory; double buffered by
-        // item parity, so one named barrier per item is enough
-        uint2* mg = s_merge + (((n & 1u) * 2u + sub) << 7);
-        if (set >= 2u) mg[row] = make_uint2(gbest, gsecond);
-        asm volatile("bar.sync %0, 256;" ::"r"(1u + sub) : "memory");
-        writer = writer && set < 2u;
-        if (writer) {
-          const uint2 o = mg[row];
-          top2_insert(gbest, gsecond, o.x);
-          top2_insert(gbest, gsecond, o.y);
-        }
-      }
-      if (writer) {
+      g_item = g_end;
+      // the two sets of a sub-tile (even / odd train tiles) meet in shared memory; double buffered by
+      // item parity, so one named barrier per item is enough
+      uint2* mg = s_merge + (((n & 1u) * 2u + sub) << 7);
+      if (set >= 2u) mg[row] = make_uint2(gbest, gsecond);
+      asm volatile("bar.sync %0, 256;" ::"r"(1u + sub) : "memory");
+      if (set < 2u && row < rows_valid) {
+        const uint2 o = mg[row];
+        top2_insert(gbest, gsecond, o.x);
+        top2_insert(gbest, gsecond, o.y);
         const int qo = p.q_off[pair];
         // best-only: gsecond is not a second neighbour (the merge of the two sets above put the larger of their bests there)
         const uint32_t ob = gbest >= kKey32Pad ? kNone : gbest, os = (!TOP2 || gsecond >= kKey32Pad) ? kNone : gsecond;
@@ -1158,11 +905,6 @@ __global__ void __launch_bounds__(kI8sThreads, 1) hamming_knn2_i8s_kernel(const 
         }
       }
       ++n;
-    }
-    if (DBG && threadIdx.x == 64) {
-      p.dbg[blockIdx.x * 8 + 4] = (unsigned long long)(clock64() - e_start);
-      p.dbg[blockIdx.x * 8 + 5] = (unsigned long long)w_tfull;
-    }
     }
   }
 
@@ -1325,34 +1067,20 @@ int hamming_i8_timing(int enable, float* last_ms) {
   return B2S_OK;
 }
 
-static unsigned long long* g_i8_dbg = nullptr;  // device buffer, 8 u64 per SM (diagnostics only)
-static int g_i8_mode = 0;
-void hamming_i8_set_debug(unsigned long long* dev_buf, int mode) {
-  g_i8_dbg = dev_buf;
-  g_i8_mode = mode;
-}
-
 constexpr size_t kI8SmemBytes =
     (size_t)(2 + kI8Stages) * kI8TileBytes + 2 * kI8ChunkBytes + 8 * (2 * kI8Stages + 9) + 128 * sizeof(uint2);
 
 int hamming_merge_launch(const uint2* partial, int total_nq, int t_split, uint32_t* fwd_best, uint32_t* fwd_second,
                          cudaStream_t st);  // hamming_popc.cu
 
-// Work decomposition of the single-product kernel: sub-tiles per item and the train-axis split.
+// Work decomposition of the single-product kernel: the train-axis split.
 // A lone 10 000 x 10 000 pair has 40 (pair, 256-query block) items for 148 SMs, a lone 2000 x 2000 pair 8:
 // the train axis is then cut into t_split pieces (merged afterwards on the packed keys, like K1's t_split) so
 // that whole waves of items cover the machine.
-struct I8sPlan {
-  int subs, t_split;
-};
-static I8sPlan plan_i8s(int n_pairs, int max_nq, int max_nt, int t_split_req, int mode) {
+static int plan_i8s(int n_pairs, int max_nq, int max_nt, int t_split_req) {
   const int qt = (max_nq + kI8Tile - 1) / kI8Tile, tt = (max_nt + kI8Tile - 1) / kI8Tile;
   const long sms = sm_count();
-  // 4 sub-tiles per item halve the L2 -> SM operand traffic but measured 8 % SLOWER on every BASELINE shape
-  // (0.276 vs 0.254 ms on the 296-pair batch, profiles/r02_k2s_plans.txt): the kernel is bound by the epilogue's
-  // ALU work, not by L2, and the 2-stage train ring prefetches less.  Kept selectable (mode bit 64) for A/B runs.
-  const int subs = ((mode & 64) && !(mode & 16)) ? 4 : 2;
-  const long base = (long)n_pairs * ((qt + subs - 1) / subs);
+  const long base = (long)n_pairs * ((qt + kI8sSubTiles - 1) / kI8sSubTiles);
   int ts = 1;
   if (t_split_req > 0) {
     ts = t_split_req;
@@ -1370,7 +1098,7 @@ static I8sPlan plan_i8s(int n_pairs, int max_nq, int max_nt, int t_split_req, in
   }
   if (ts > tt) ts = tt;
   if (ts < 1) ts = 1;
-  return I8sPlan{subs, ts};
+  return ts;
 }
 
 static size_t partial_bytes(int total_nq, int t_split) {
@@ -1379,9 +1107,8 @@ static size_t partial_bytes(int total_nq, int t_split) {
 
 size_t hamming_i8_workspace_bytes(int n_pairs, int total_nq, int max_nq, int max_nt, int t_split) {
   const size_t qt = (size_t)((max_nq + kI8Tile - 1) / kI8Tile), tt = (size_t)((max_nt + kI8Tile - 1) / kI8Tile);
-  const I8sPlan pl = plan_i8s(n_pairs, max_nq, max_nt, t_split, 0);
   // sized for the largest layout (unified 18-chunk tiles on both sides) + the partial top-2 of a train-axis split
-  return (size_t)n_pairs * (qt + tt) * kI8sQTileBytes + partial_bytes(total_nq, pl.t_split);
+  return (size_t)n_pairs * (qt + tt) * kI8sQTileBytes + partial_bytes(total_nq, plan_i8s(n_pairs, max_nq, max_nt, t_split));
 }
 
 // every key starts as "none".  Three separate memset nodes on purpose: ONE 7 MB memset over the (often
@@ -1399,42 +1126,37 @@ static int clear_keys(uint32_t* fwd_best, uint32_t* fwd_second, uint32_t* bwd_be
 
 // the single-product kernel: picks the instantiation, opts into its shared memory (per launch: the
 // attribute is per device, and a process may drive several), brackets it with the timing events
-template <int EPI, bool DBG, int SUBS, bool TOP2 = true>
+template <bool TOP2>
 static int launch_i8s_inst(const I8Params& p, int grid, cudaStream_t st) {
   static bool attr_set[64] = {false};   // one flag array per instantiation
   if (first_use_on_device(attr_set))
-    B2S_CUDA(cudaFuncSetAttribute(hamming_knn2_i8s_kernel<EPI, DBG, SUBS, TOP2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  (int)I8sCfg<SUBS>::kSmem));
-  hamming_knn2_i8s_kernel<EPI, DBG, SUBS, TOP2><<<grid, kI8sThreads, I8sCfg<SUBS>::kSmem, st>>>(p);
+    B2S_CUDA(cudaFuncSetAttribute(hamming_knn2_i8s_kernel<TOP2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  (int)kI8sSmemBytes));
+  hamming_knn2_i8s_kernel<TOP2><<<grid, kI8sThreads, kI8sSmemBytes, st>>>(p);
   return B2S_OK;
 }
-static int g_i8_last_plan[3] = {0, 0, 0};   // subs, t_split, grid of the most recent launch (diagnostics)
+static int g_i8_last_plan[2] = {0, 0};   // t_split, grid of the most recent launch (diagnostics)
 void hamming_i8_last_plan(int* subs, int* t_split, int* grid) {
-  if (subs) *subs = g_i8_last_plan[0];
-  if (t_split) *t_split = g_i8_last_plan[1];
-  if (grid) *grid = g_i8_last_plan[2];
+  if (subs) *subs = kI8sSubTiles;
+  if (t_split) *t_split = g_i8_last_plan[0];
+  if (grid) *grid = g_i8_last_plan[1];
 }
-static int launch_i8s(I8Params& p, const I8sPlan& pl, int total_nq, uint8_t* partial_ws, bool need_second, cudaStream_t st) {
-  p.t_split = pl.t_split;
+static int launch_i8s(I8Params& p, int t_split, int total_nq, uint8_t* partial_ws, bool need_second, cudaStream_t st) {
+  p.t_split = t_split;
   p.total_nq = total_nq;
-  p.partial = pl.t_split > 1 ? reinterpret_cast<uint2*>(partial_ws) : nullptr;
-  if (pl.t_split > 1)   // parts that own no train tile of a short pair still report "none"
-    B2S_CUDA(cudaMemsetAsync(partial_ws, 0xFF, sizeof(uint2) * (size_t)total_nq * pl.t_split, st));
-  const long items = (long)((p.q_tiles + pl.subs - 1) / pl.subs) * p.n_pairs * pl.t_split;
+  p.partial = t_split > 1 ? reinterpret_cast<uint2*>(partial_ws) : nullptr;
+  if (t_split > 1)   // parts that own no train tile of a short pair still report "none"
+    B2S_CUDA(cudaMemsetAsync(partial_ws, 0xFF, sizeof(uint2) * (size_t)total_nq * t_split, st));
+  const long items = (long)((p.q_tiles + kI8sSubTiles - 1) / kI8sSubTiles) * p.n_pairs * t_split;
   const int grid = (int)(items < (long)sm_count() ? items : (long)sm_count());
-  g_i8_last_plan[0] = pl.subs, g_i8_last_plan[1] = pl.t_split, g_i8_last_plan[2] = grid;
+  g_i8_last_plan[0] = t_split, g_i8_last_plan[1] = grid;
   if (g_i8_timing) B2S_CUDA(cudaEventRecord(g_i8_ev[0], st));
-  int rc;
-  if (p.mode & 16) rc = launch_i8s_inst<0, true, 2>(p, grid, st);            // 32x32b epilogue (A/B partner)
-  else if (!need_second && pl.subs == 2 && !p.dbg) rc = launch_i8s_inst<1, false, 2, false>(p, grid, st);   // best neighbour only
-  else if (pl.subs == 4) rc = p.dbg ? launch_i8s_inst<1, true, 4>(p, grid, st) : launch_i8s_inst<1, false, 4>(p, grid, st);
-  else rc = p.dbg ? launch_i8s_inst<1, true, 2>(p, grid, st) : launch_i8s_inst<1, false, 2>(p, grid, st);
-  if (rc) return rc;
+  if (int rc = need_second ? launch_i8s_inst<true>(p, grid, st) : launch_i8s_inst<false>(p, grid, st)) return rc;
   B2S_CUDA(cudaGetLastError());
   if (g_i8_timing) B2S_CUDA(cudaEventRecord(g_i8_ev[1], st));
   note_launch();
-  if (pl.t_split > 1) {
-    if (int rc2 = hamming_merge_launch(p.partial, total_nq, pl.t_split, p.fwd_best, p.fwd_second, st)) return rc2;
+  if (t_split > 1) {
+    if (int rc2 = hamming_merge_launch(p.partial, total_nq, t_split, p.fwd_best, p.fwd_second, st)) return rc2;
     // best-only: the merge folded the parts' BEST keys into fwd_second; that is not a second neighbour
     if (!need_second) B2S_CUDA(cudaMemsetAsync(p.fwd_second, 0xFF, sizeof(uint32_t) * (size_t)total_nq, st));
   }
@@ -1450,21 +1172,20 @@ int hamming_i8_launch(const uint8_t* q, const uint8_t* t, const int32_t* q_off, 
   if (total_nq == 0 || total_nt == 0 || max_nq == 0 || max_nt == 0) return B2S_OK;
   const int qt = (max_nq + kI8Tile - 1) / kI8Tile, tt = (max_nt + kI8Tile - 1) / kI8Tile;
   const size_t tiles_bytes = (size_t)n_pairs * (qt + tt) * kI8sQTileBytes;
-  I8sPlan pl = plan_i8s(n_pairs, max_nq, max_nt, single ? t_split : 1, g_i8_mode);
-  while (pl.t_split > 1 && tiles_bytes + partial_bytes(total_nq, pl.t_split) > workspace_bytes) --pl.t_split;  // shrink rather than fail
-  const size_t need = tiles_bytes + partial_bytes(total_nq, single ? pl.t_split : 1);
+  int split = plan_i8s(n_pairs, max_nq, max_nt, single ? t_split : 1);
+  while (split > 1 && tiles_bytes + partial_bytes(total_nq, split) > workspace_bytes) --split;  // shrink rather than fail
+  const size_t need = tiles_bytes + partial_bytes(total_nq, single ? split : 1);
   B2S_REQUIRE(workspace != nullptr && workspace_bytes >= need,
               "i8 variant needs %zu workspace bytes (b2s_hamming_workspace_bytes_v), got %zu", need, workspace_bytes);
   B2S_REQUIRE(((uintptr_t)workspace & 127u) == 0, "workspace must be 128-byte aligned");
-  const bool unified = single && !(g_i8_mode & 16);   // the 16x256b epilogue reads unified tiles (layout 3)
   const int q_units = (single ? kI8Chunks + 1 : kI8Chunks) * kI8Tile;
   uint8_t* qx = static_cast<uint8_t*>(workspace);
   uint8_t* tx = qx + (size_t)n_pairs * qt * q_units * 16;
-  expand_pm8_kernel<<<dim3(qt, n_pairs), 128, 0, st>>>(q, q_off, q_src, qt, 0, unified ? 3 : single ? 1 : 0,
-                                                                               reinterpret_cast<uint4*>(qx), nullptr, nullptr);
+  expand_pm8_kernel<<<dim3(qt, n_pairs), 128, 0, st>>>(q, q_off, q_src, qt, 0, single != 0, reinterpret_cast<uint4*>(qx),
+                                                       nullptr, nullptr);
   B2S_CUDA(cudaGetLastError());
-  expand_pm8_kernel<<<dim3(tt, n_pairs), 128, 0, st>>>(t, t_off, t_src, tt, 1, unified ? 3 : single ? 2 : 0,
-                                                                                reinterpret_cast<uint4*>(tx), nullptr, nullptr);
+  expand_pm8_kernel<<<dim3(tt, n_pairs), 128, 0, st>>>(t, t_off, t_src, tt, 1, single != 0, reinterpret_cast<uint4*>(tx),
+                                                       nullptr, nullptr);
   B2S_CUDA(cudaGetLastError());
   note_launch(2);
   I8Params p;
@@ -1480,12 +1201,10 @@ int hamming_i8_launch(const uint8_t* q, const uint8_t* t, const int32_t* q_off, 
   p.n_pairs = n_pairs;
   p.q_xt = nullptr;
   p.t_xt = nullptr;
-  p.dbg = g_i8_dbg;
-  p.mode = g_i8_mode;
   p.t_split = 1;
   p.total_nq = total_nq;
   p.partial = nullptr;
-  if (single) return launch_i8s(p, pl, total_nq, static_cast<uint8_t*>(workspace) + tiles_bytes, need_second != 0, st);
+  if (single) return launch_i8s(p, split, total_nq, static_cast<uint8_t*>(workspace) + tiles_bytes, need_second != 0, st);
   static bool attr_set[64] = {false};
   if (first_use_on_device(attr_set))
     B2S_CUDA(cudaFuncSetAttribute(hamming_knn2_i8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kI8SmemBytes));
@@ -1500,12 +1219,11 @@ int hamming_i8_launch(const uint8_t* q, const uint8_t* t, const int32_t* q_off, 
 }
 
 size_t hamming_i8_shared_workspace_bytes(int total_tiles, int n_pairs, int total_nq, int max_nq, int max_nt, int t_split) {
-  const I8sPlan pl = plan_i8s(n_pairs, max_nq, max_nt, t_split, 0);
-  return (size_t)total_tiles * kI8sQTileBytes + partial_bytes(total_nq, pl.t_split);
+  return (size_t)total_tiles * kI8sQTileBytes + partial_bytes(total_nq, plan_i8s(n_pairs, max_nq, max_nt, t_split));
 }
 
 // Batches whose pairs share descriptor blocks (frames): every block is expanded ONCE into unified
-// tiles, the pairs address them through q_xtile / t_xtile.  Single-product kernel, 16x256b epilogue.
+// tiles, the pairs address them through q_xtile / t_xtile.  Single-product kernel.
 int hamming_i8_shared_launch(const uint8_t* desc, const int32_t* blk_row0, const int32_t* blk_rows,
                              const int32_t* blk_tile0, int n_blocks, int total_tiles, int max_block_rows,
                              const int32_t* q_xtile, const int32_t* t_xtile, const int32_t* q_off, const int32_t* t_off,
@@ -1516,16 +1234,16 @@ int hamming_i8_shared_launch(const uint8_t* desc, const int32_t* blk_row0, const
   if (int rc = clear_keys(fwd_best, fwd_second, bwd_best, total_nq, total_nt, st)) return rc;
   if (total_nq == 0 || total_nt == 0 || max_nq == 0 || max_nt == 0 || n_blocks == 0) return B2S_OK;
   const size_t tiles_bytes = (size_t)total_tiles * kI8sQTileBytes;
-  I8sPlan pl = plan_i8s(n_pairs, max_nq, max_nt, t_split, g_i8_mode & ~16);
-  while (pl.t_split > 1 && tiles_bytes + partial_bytes(total_nq, pl.t_split) > workspace_bytes) --pl.t_split;
-  const size_t need = tiles_bytes + partial_bytes(total_nq, pl.t_split);
+  int split = plan_i8s(n_pairs, max_nq, max_nt, t_split);
+  while (split > 1 && tiles_bytes + partial_bytes(total_nq, split) > workspace_bytes) --split;
+  const size_t need = tiles_bytes + partial_bytes(total_nq, split);
   B2S_REQUIRE(workspace != nullptr && workspace_bytes >= need,
               "shared-block Hamming needs %zu workspace bytes (b2s_hamming_shared_workspace_bytes), got %zu", need,
               workspace_bytes);
   B2S_REQUIRE(((uintptr_t)workspace & 127u) == 0, "workspace must be 128-byte aligned");
   const int bt = (max_block_rows + kI8Tile - 1) / kI8Tile;
   uint8_t* x = static_cast<uint8_t*>(workspace);
-  expand_pm8_kernel<<<dim3(bt, n_blocks), 128, 0, st>>>(desc, nullptr, blk_row0, 0, 0, 3, reinterpret_cast<uint4*>(x),
+  expand_pm8_kernel<<<dim3(bt, n_blocks), 128, 0, st>>>(desc, nullptr, blk_row0, 0, 0, true, reinterpret_cast<uint4*>(x),
                                                        blk_rows, blk_tile0);
   B2S_CUDA(cudaGetLastError());
   note_launch();
@@ -1542,9 +1260,7 @@ int hamming_i8_shared_launch(const uint8_t* desc, const int32_t* blk_row0, const
   p.n_pairs = n_pairs;
   p.q_xt = q_xtile;
   p.t_xt = t_xtile;
-  p.dbg = g_i8_dbg;
-  p.mode = g_i8_mode & ~16;
-  return launch_i8s(p, pl, total_nq, x + tiles_bytes, need_second != 0, st);
+  return launch_i8s(p, split, total_nq, x + tiles_bytes, need_second != 0, st);
 }
 
 }  // namespace b2s

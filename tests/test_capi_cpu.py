@@ -69,7 +69,7 @@ def test_sass_is_blackwell_native():
         hits = [k for k in funcs if all(n in k for n in needles)]
         assert hits, needles
         return "\n".join(funcs[hits[0]])
-    k2s = body("hamming_knn2_i8s_kernel", "ILi1ELb0ELi2E")          # <EPI = 1, DBG = false, SUBS = 2>: the shipped instantiation
+    k2s = body("hamming_knn2_i8s_kernel", "ILb1E")                  # <TOP2 = true>: the kNN-2 instantiation
     assert k2s.count("UTCIMMA") >= 18 and "LDTM" in k2s and "UTCBAR" in k2s and "UBLKCP" in k2s
     assert "VIMNMX3" in k2s and "VIADDMNMX" in k2s                  # the packed 16-bit key epilogue
     k2 = body("hamming_knn2_i8_kernel")

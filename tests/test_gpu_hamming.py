@@ -281,7 +281,7 @@ def test_shared_block_path_equals_per_pair_expansion():
         assert np.array_equal(bw[to:to + len(t)], rw), p
 
 
-# ---- K2s work decomposition: 2 / 4 query sub-tiles per item x train-axis split ----------
+# ---- K2s work decomposition: 2 query sub-tiles per item x train-axis split ----------
 
 def _plan(lib):
     import ctypes as C
@@ -290,49 +290,43 @@ def _plan(lib):
     return tuple(x.value for x in v)
 
 
-@pytest.mark.parametrize("force", [32, 64], ids=["2_subtiles", "4_subtiles"])
-@pytest.mark.parametrize("t_split", [0, 1, 2, 3, 7, 64])
-def test_k2s_decompositions_are_bit_exact(hg, force, t_split):
-    """Every (sub-tiles per item, train split) plan of the single-product kernel gives the POPC kernel's /
-    the oracle's keys: golden tie-heavy cases, ragged batches with empty sides and tile-edge sizes, and a
-    lone 2000 x 2000 pair (the drop-in call: 8 or 4 work items without the split)."""
+@pytest.mark.parametrize("t_split", [0, 1, 2, 3, 4, 5, 6, 7, 8, 11, 16, 64])
+def test_k2s_decompositions_are_bit_exact(hg, t_split):
+    """Every train-split plan of the single-product kernel gives the POPC kernel's / the oracle's keys:
+    golden tie-heavy cases, ragged batches with empty sides and tile-edge sizes, and a lone 2000 x 2000
+    pair (the drop-in call: 8 work items without the split)."""
     from b200slam import _capi
     from b200slam.frontend import HammingMatcher
     lib = _capi.load_library()
-    lib.b2s_hamming_i8_debug(None, force)
-    try:
-        m = HammingMatcher(variant=_capi.VARIANT_I8MMA1, t_split=t_split)
-        k1 = HammingMatcher(variant=_capi.VARIANT_POPC)
-        names = ["noisy_2000x2000", "tie_w2_127x129", "orb_real_0", "duplicates_70x70", "tie_w32_300x257", "noisy_640x33"]
-        rng = np.random.default_rng(5 + t_split)
-        sizes = [(int(rng.integers(1, 1200)), int(rng.integers(1, 1200))) for _ in range(6)] + [(0, 9), (9, 0), (513, 129), (1, 1025), (1025, 1)]
-        qs = [_pad(hg[f"{n}/q"]) for n in names] + [rng.integers(0, 4, (a, 32), dtype=np.uint8) for a, _ in sizes]
-        ts = [_pad(hg[f"{n}/t"]) for n in names] + [rng.integers(0, 4, (b, 32), dtype=np.uint8) for _, b in sizes]
-        got, want = m.knn2_pairs(qs, ts), k1.knn2_pairs(qs, ts)
-        subs, ts_used, _ = _plan(lib)
-        assert subs == (2 if force == 32 else 4)
-        if t_split > 0:
-            assert ts_used == min(t_split, (max(len(t) for t in ts) + 127) // 128)
-        for i, ((fb, fs, bb), (wb, ws, wbb)) in enumerate(zip(got, want)):
-            np.testing.assert_array_equal(fb, wb, err_msg=str(i))
-            np.testing.assert_array_equal(fs, ws, err_msg=str(i))
-            np.testing.assert_array_equal(bb, wbb, err_msg=str(i))
-        # one lone pair, against the oracle
-        (fb, fs, bb), = m.knn2_pairs([qs[0]], [ts[0]])
-        b, s, bw = ho.packed_keys(qs[0], ts[0])
-        np.testing.assert_array_equal(fb, b)
-        np.testing.assert_array_equal(fs, s)
-        np.testing.assert_array_equal(bb, bw)
-        if t_split == 0:
-            assert _plan(lib)[1] > 1, "a lone pair must be split along the train axis"
-    finally:
-        lib.b2s_hamming_i8_debug(None, 0)
+    m = HammingMatcher(variant=_capi.VARIANT_I8MMA1, t_split=t_split)
+    k1 = HammingMatcher(variant=_capi.VARIANT_POPC)
+    names = ["noisy_2000x2000", "tie_w2_127x129", "orb_real_0", "duplicates_70x70", "tie_w32_300x257", "noisy_640x33"]
+    rng = np.random.default_rng(5 + t_split)
+    sizes = [(int(rng.integers(1, 1200)), int(rng.integers(1, 1200))) for _ in range(6)] + [(0, 9), (9, 0), (513, 129), (1, 1025), (1025, 1)]
+    qs = [_pad(hg[f"{n}/q"]) for n in names] + [rng.integers(0, 4, (a, 32), dtype=np.uint8) for a, _ in sizes]
+    ts = [_pad(hg[f"{n}/t"]) for n in names] + [rng.integers(0, 4, (b, 32), dtype=np.uint8) for _, b in sizes]
+    got, want = m.knn2_pairs(qs, ts), k1.knn2_pairs(qs, ts)
+    subs, ts_used, _ = _plan(lib)
+    assert subs == 2
+    if t_split > 0:
+        assert ts_used == min(t_split, (max(len(t) for t in ts) + 127) // 128)
+    for i, ((fb, fs, bb), (wb, ws, wbb)) in enumerate(zip(got, want)):
+        np.testing.assert_array_equal(fb, wb, err_msg=str(i))
+        np.testing.assert_array_equal(fs, ws, err_msg=str(i))
+        np.testing.assert_array_equal(bb, wbb, err_msg=str(i))
+    # one lone pair, against the oracle
+    (fb, fs, bb), = m.knn2_pairs([qs[0]], [ts[0]])
+    b, s, bw = ho.packed_keys(qs[0], ts[0])
+    np.testing.assert_array_equal(fb, b)
+    np.testing.assert_array_equal(fs, s)
+    np.testing.assert_array_equal(bb, bw)
+    if t_split == 0:
+        assert _plan(lib)[1] > 1, "a lone pair must be split along the train axis"
 
 
-@pytest.mark.parametrize("force", [32, 64], ids=["2_subtiles", "4_subtiles"])
-@pytest.mark.parametrize("t_split", [0, 3])
-def test_k2s_shared_blocks_with_split(force, t_split):
-    """The shared-block entry (frames expanded once) under every decomposition, ragged frame sequence."""
+@pytest.mark.parametrize("t_split", [0, 1, 3, 7])
+def test_k2s_shared_blocks_with_split(t_split):
+    """The shared-block entry (frames expanded once) with and without a train split, ragged frame sequence."""
     import torch
     from b200slam import _capi
     from b200slam.frontend import HammingMatcher, sequence_batch
@@ -345,11 +339,8 @@ def test_k2s_shared_blocks_with_split(force, t_split):
     dev = torch.from_numpy(desc).cuda()
     kp = torch.zeros((F * N, 2), dtype=torch.float32, device="cuda")
     b = sequence_batch(dev, kp, counts, 0, F - 1, N)
-    lib.b2s_hamming_i8_debug(None, force)
-    try:
-        got = HammingMatcher(variant=_capi.VARIANT_I8MMA1, t_split=t_split).knn2(b)
-    finally:
-        lib.b2s_hamming_i8_debug(None, 0)
+    got = HammingMatcher(variant=_capi.VARIANT_I8MMA1, t_split=t_split).knn2(b)
+    assert _plan(lib)[0] == 2
     popc = HammingMatcher(variant=_capi.VARIANT_POPC).knn2(b)
     for name in ("fwd_best", "fwd_second", "bwd_best"):
         assert np.array_equal(getattr(got, name).cpu().numpy(), getattr(popc, name).cpu().numpy()), name

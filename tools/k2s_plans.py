@@ -1,5 +1,5 @@
 """A/B of the K2s work decompositions (GPU): kernel-only time (library events) and clk per 128x128 tile pair
-for 2 / 4 query sub-tiles per item and train-axis splits, on the BASELINE shapes.
+for train-axis splits, on the BASELINE shapes.
 Usage: python tools/k2s_plans.py"""
 import ctypes as C
 import sys
@@ -63,16 +63,13 @@ def plan():
 def report(name, batch, nq, nt, pairs, splits=(0,)):
     tile_pairs = pairs * ((nq + 127) // 128) * ((nt + 127) // 128)
     ops = 2.0 * 256 * nq * nt * pairs
-    for force, label in ((32, "2 sub-tiles"), (64, "4 sub-tiles"), (0, "auto")):
-        for ts in splits:
-            lib.b2s_hamming_i8_debug(None, force)
-            m = HammingMatcher(variant=_capi.VARIANT_I8MMA1, t_split=ts)
-            k, call = kernel_ms(m, batch)
-            subs, tsu, grid = plan()
-            gcall = graph_call_ms(m, batch)
-            lib.b2s_hamming_i8_debug(None, 0)
-            print(f"{name:28s} {label:12s} t_split {ts:2d} -> plan subs {subs} t_split {tsu:2d} grid {grid:3d}: kernel(events, eager) {k:.4f} ms "
-                  f"call(eager) {call:.4f} ms  call(graph x20) {gcall:.4f} ms = {ops / (gcall * 1e-3) / 1e15:.3f} POP/s whole call", flush=True)
+    for ts in splits:
+        m = HammingMatcher(variant=_capi.VARIANT_I8MMA1, t_split=ts)
+        k, call = kernel_ms(m, batch)
+        subs, tsu, grid = plan()
+        gcall = graph_call_ms(m, batch)
+        print(f"{name:28s} t_split {ts:2d} -> plan subs {subs} t_split {tsu:2d} grid {grid:3d}: kernel(events, eager) {k:.4f} ms "
+              f"call(eager) {call:.4f} ms  call(graph x20) {gcall:.4f} ms = {ops / (gcall * 1e-3) / 1e15:.3f} POP/s whole call", flush=True)
 
 
 rng = np.random.default_rng(0)

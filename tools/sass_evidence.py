@@ -64,10 +64,10 @@ def main():
     for short, c, _ in sorted(rows, key=lambda r: -r[1]["total"]):
         md.append(f"| `{short}` | {c['total']} | " + " | ".join(str(c[o]) if c[o] else "" for o in OPS) + " |")
     # trimmed listing of the shipped Hamming kernel
-    target = [r for r in rows if "hamming_knn2_i8s_kernel<1, false, 2, true>" in r[0]]
+    target = [r for r in rows if "hamming_knn2_i8s_kernel<true>" in r[0]]
     if target:
         _, _, mangled = target[0]
-        md += ["", "## `hamming_knn2_i8s_kernel<1, false, 2, true>` (shipped) — every tensor-core / TMEM / bulk-copy line", "", "```"]
+        md += ["", "## `hamming_knn2_i8s_kernel<true>` (shipped) — every tensor-core / TMEM / bulk-copy line", "", "```"]
         md += [l.split("*/", 1)[0].strip() + "*/ " + re.sub(r"\s*/\*.*", "", l.split("*/", 1)[1]).strip()
                for l in ks[mangled] if re.search(r"UTCIMMA|LDTM|UTCBAR|UBLKCP|UTCATOM|ELECT", l)]
         md += ["```"]
