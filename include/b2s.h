@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define B2S_ABI_VERSION 4
+#define B2S_ABI_VERSION 5
 #define B2S_IDX_BITS 22
 #define B2S_IDX_MASK ((1u << B2S_IDX_BITS) - 1u)
 #define B2S_NONE_KEY 0xFFFFFFFFu
@@ -179,8 +179,12 @@ int b2s_ransac_score_batched(const float* corr, const int32_t* c_off, const int3
  *                              (th in the units of the points; th_per_pair optional);
  * b2s_homography_select        replaces the strict-improvement / 0.8 n early-exit bookkeeping, :207-211,
  *                              and writes the winner's inlier mask. */
+/* samples_in == NULL: the device draws 4 distinct indices from (seed, id(p), h) with id(p) = pair_ids[p] (device int32,
+ * optional) or pair_id0 + p, the pair's GLOBAL id, as b2s_eight_point_batched does: a pair draws the same samples on
+ * whichever rank / batch position it is processed (pair_ids = NULL, pair_id0 = 0: id(p) = p). */
 int b2s_homography_dlt_batched(const float* corr, const int32_t* c_off, const int32_t* c_count, int n_pairs, int H,
-                               const int32_t* samples_in, uint64_t seed, int32_t* samples_out, double* H_out, void* stream);
+                               const int32_t* samples_in, uint64_t seed, const int32_t* pair_ids, int pair_id0,
+                               int32_t* samples_out, double* H_out, void* stream);
 int b2s_homography_score_batched(const float* corr, const int32_t* c_off, const int32_t* c_count, int n_pairs,
                                  const double* Hm, int H, double th, const double* th_per_pair, int32_t* counts,
                                  void* stream);
@@ -299,6 +303,17 @@ int b2s_ransac_select(const int32_t* counts, const float* corr, const int32_t* c
  * pair_id0 + p; src_pair (optional, n_records int32): record r describes pair src_pair[r] (-1 = empty
  * slot) and best_h / best_count / R / t are then indexed by r (ranked candidates, b2s_rank_pairs). */
 size_t b2s_record_bytes(int max_matches);
+/* Pose record: the answer of the robust pose estimator (b2s_robust_pose_decide with a record sink) appended to a result
+ * record, so that every offset of the record above stays where it is:
+ *   pose record = record of b2s_record_bytes(S) bytes | b2s_pose_result (B2S_POSE_RESULT_BYTES = 200) | 56 zero bytes
+ * b2s_pose_record_bytes(S) = b2s_record_bytes(S) + B2S_POSE_BLOCK_BYTES (S = 500: 3584 + 256 = 3840 bytes).  The
+ * header of a pose record: n_matches = the selection count (-1 on overflow), best_h = the SELECTED model's RANSAC winner
+ * (e_best_h or h_best_h of the result; -1 for an error outcome), inlier_count = result.inliers, pair_id = pair_id0 + p,
+ * R | t = the result's R and normalised t as float32 (zero for an error outcome); inlier[S] = the selected model's
+ * flags (zero past n_matches, and all zero for an error outcome).  A record slot that holds no pair (the padding of a
+ * sharded gather buffer) has pair_id -1 and, in a pose record, outcome -1. */
+#define B2S_POSE_BLOCK_BYTES 256
+size_t b2s_pose_record_bytes(int max_matches);
 int b2s_pack_records(const int32_t* count, const int32_t* count_total, const int32_t* best_h, const int32_t* best_count,
                      const int32_t* out_q, const int32_t* out_t, const int32_t* out_d, const uint8_t* inlier_mask,
                      const double* R, const double* t, const int32_t* pair_ids, const int32_t* src_pair, int n_records,
@@ -402,9 +417,15 @@ typedef struct b2s_pose_result {
 #ifdef __cplusplus
 static_assert(sizeof(b2s_robust_pose_config) == B2S_ROBUST_POSE_CONFIG_BYTES, "b2s_robust_pose_config layout");
 static_assert(sizeof(b2s_pose_result) == B2S_POSE_RESULT_BYTES, "b2s_pose_result layout");
+static_assert(offsetof(b2s_pose_result, inlier_ratio) == 48 && offsetof(b2s_pose_result, threshold) == 96 &&
+              offsetof(b2s_pose_result, R) == 104 && offsetof(b2s_pose_result, t) == 176, "b2s_pose_result offsets");
+static_assert(B2S_POSE_BLOCK_BYTES >= B2S_POSE_RESULT_BYTES && B2S_POSE_BLOCK_BYTES % 64 == 0, "pose block");
 #else
 _Static_assert(sizeof(b2s_robust_pose_config) == B2S_ROBUST_POSE_CONFIG_BYTES, "b2s_robust_pose_config layout");
 _Static_assert(sizeof(b2s_pose_result) == B2S_POSE_RESULT_BYTES, "b2s_pose_result layout");
+_Static_assert(offsetof(b2s_pose_result, inlier_ratio) == 48 && offsetof(b2s_pose_result, threshold) == 96 &&
+               offsetof(b2s_pose_result, R) == 104 && offsetof(b2s_pose_result, t) == 176, "b2s_pose_result offsets");
+_Static_assert(B2S_POSE_BLOCK_BYTES >= B2S_POSE_RESULT_BYTES && B2S_POSE_BLOCK_BYTES % 64 == 0, "pose block");
 #endif
 
 /* Median displacement per pair: np.median(np.linalg.norm(pts2[sel] - pts1[sel], axis=1)) on the float32
@@ -437,6 +458,17 @@ int b2s_robust_pose_decide(const int32_t* c_off, const int32_t* c_count, int n_p
                            const int32_t* h_best_h, const int32_t* h_inliers, const uint8_t* h_mask, const double* H_fit,
                            const double* Kinv_host, const b2s_robust_pose_config* cfg, int n_cfg,
                            b2s_pose_result* results, uint8_t* out_mask, int mask_stride, void* stream);
+/* The same decision, and the same kernel launch, that also writes every pair's POSE record (b2s_pose_record_bytes
+ * above) from the sink's selection outputs and its own result and flags: no extra launch at the end of a robust step.
+ * sink NULL (or records NULL) = b2s_robust_pose_decide.  The sink needs record_bytes >= b2s_pose_record_bytes(stride),
+ * a multiple of 16, 16-byte aligned records, and the compact selection layout (pair p at p * stride). */
+int b2s_robust_pose_decide_records(const int32_t* c_off, const int32_t* c_count, int n_pairs, const int32_t* e_best_h,
+                                   const int32_t* e_inliers, const uint8_t* e_mask, const double* e_R, const double* e_t,
+                                   const int32_t* e_votes, const float* e_median, const float* all_median, const double* th,
+                                   const int32_t* h_best_h, const int32_t* h_inliers, const uint8_t* h_mask,
+                                   const double* H_fit, const double* Kinv_host, const b2s_robust_pose_config* cfg, int n_cfg,
+                                   b2s_pose_result* results, uint8_t* out_mask, int mask_stride, const b2s_record_sink* sink,
+                                   void* stream);
 
 /* ---- measurement helper ----------------------------------------------------------
  * Saturates one SM pipe with independent instructions to measure its rate:

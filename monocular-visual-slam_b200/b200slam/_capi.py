@@ -21,7 +21,7 @@ IDX_MASK = (1 << IDX_BITS) - 1
 NONE_KEY = 0xFFFFFFFF
 DESC_BYTES = 32
 SELECT_MAX_QUERIES = 32768
-ABI_VERSION = 4
+ABI_VERSION = 5
 VARIANT_POPC = 0
 VARIANT_I8MMA = 1
 VARIANT_I8MMA1 = 2
@@ -82,6 +82,8 @@ def _declare(lib):
                                        vp, vp, vp, vp, i32, vp, vp, vp, vp, vp, vp, vp]
     lib.b2s_record_bytes.restype = sz
     lib.b2s_record_bytes.argtypes = [i32]
+    lib.b2s_pose_record_bytes.restype = sz
+    lib.b2s_pose_record_bytes.argtypes = [i32]
     lib.b2s_pack_records.restype = i32
     lib.b2s_pack_records.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, vp, sz, vp]
     lib.b2s_rank_pairs.restype = i32
@@ -95,7 +97,7 @@ def _declare(lib):
     lib.b2s_ransac_score_tc.restype = i32
     lib.b2s_ransac_score_tc.argtypes = [vp, vp, vp, i32, i32, vp, i32, dbl, vp, vp, vp, sz, vp, vp, i32, vp, vp]
     lib.b2s_homography_dlt_batched.restype = i32
-    lib.b2s_homography_dlt_batched.argtypes = [vp, vp, vp, i32, i32, vp, u64, vp, vp, vp]
+    lib.b2s_homography_dlt_batched.argtypes = [vp, vp, vp, i32, i32, vp, u64, vp, i32, vp, vp, vp]
     lib.b2s_homography_score_batched.restype = i32
     lib.b2s_homography_score_batched.argtypes = [vp, vp, vp, i32, vp, i32, dbl, vp, vp, vp]
     lib.b2s_homography_select.restype = i32
@@ -124,6 +126,9 @@ def _declare(lib):
     lib.b2s_refit_homography_batched.argtypes = [vp, vp, vp, vp, i32, vp, vp, vp]
     lib.b2s_robust_pose_decide.restype = i32
     lib.b2s_robust_pose_decide.argtypes = [vp, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, i32, vp]
+    lib.b2s_robust_pose_decide_records.restype = i32
+    lib.b2s_robust_pose_decide_records.argtypes = [vp, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, i32,
+                                                   vp, vp]
     lib.b2s_hamming_kernel_timing.restype = i32
     lib.b2s_hamming_kernel_timing.argtypes = [i32, C.POINTER(C.c_float)]
     lib.b2s_mma_microbench.restype = i32
@@ -143,8 +148,9 @@ EXPORTS = (
     "b2s_hamming_kernel_timing", "b2s_ransac_score_tc_workspace_bytes", "b2s_ransac_score_tc",
     "b2s_homography_dlt_batched", "b2s_homography_score_batched", "b2s_homography_select", "b2s_decompose_essential_batched", "b2s_refit_essential_batched", "b2s_pose_pick", "b2s_five_point_batched",
     "b2s_bow_histogram_batched", "b2s_bow_cosine", "b2s_hamming_shared_workspace_bytes", "b2s_hamming_knn2_shared", "b2s_hamming_last_plan",
-    "b2s_record_bytes", "b2s_pack_records", "b2s_rank_pairs", "b2s_ransac_winner_workspace_bytes", "b2s_ransac_winner_batched",
+    "b2s_record_bytes", "b2s_pose_record_bytes", "b2s_pack_records", "b2s_rank_pairs", "b2s_ransac_winner_workspace_bytes", "b2s_ransac_winner_batched",
     "b2s_displacement_median_batched", "b2s_refit_homography_batched", "b2s_robust_pose_decide",
+    "b2s_robust_pose_decide_records",
 )
 
 

@@ -438,6 +438,17 @@ def record_bytes(max_matches: int) -> int:
     return int(_capi.load_library().b2s_record_bytes(int(max_matches)))
 
 
+def pose_record_bytes(max_matches: int) -> int:
+    """Bytes of a pose record (include/b2s.h): a result record of record_bytes(max_matches) bytes, then the pair's
+    b2s_pose_result (200 bytes) and 56 zero bytes.  What a step with FrontendConfig.robust_pose writes per pair."""
+    return int(_capi.load_library().b2s_pose_record_bytes(int(max_matches)))
+
+
+def step_record_bytes(cfg) -> int:
+    """Record bytes per pair of a step run with `cfg` (FrontendConfig): pose records when cfg.robust_pose is set."""
+    return pose_record_bytes(cfg.max_matches) if cfg.robust_pose is not None else record_bytes(cfg.max_matches)
+
+
 def pack_records(records, sel: Selection, best_h=None, best_count=None, mask=None, R=None, t=None, *, n_records: int,
                  pair_id0: int = 0, pair_ids=None, src_pair=None, count_total=None):
     """Write one record per pair into `records` (device uint8 [n_records, record_bytes(sel.stride)], e.g. this
@@ -452,19 +463,29 @@ def pack_records(records, sel: Selection, best_h=None, best_count=None, mask=Non
     return records
 
 
-def unpack_records(buf, stride: int):
+def unpack_records(buf, stride: int, pose: bool = False):
     """Host view of a record buffer (NumPy uint8 [n, record_bytes]) -> dict of arrays: n_matches, best_h,
     inliers, pair_id (int32 [n]); R float32 [n, 3, 3]; t float32 [n, 3]; q, t_idx, d (uint16 [n, stride]);
-    inlier (uint8 [n, stride]).  Entries past n_matches are zero."""
+    inlier (uint8 [n, stride]).  Entries past n_matches are zero.  pose=True: pose records (pose_record_bytes), and
+    "robust" holds every pair's b2s_pose_result (robust_pose.POSE_RESULT_DTYPE [n]); best_h / inliers / R / t / inlier
+    are then those of the selected model."""
     a = np.ascontiguousarray(np.asarray(buf, dtype=np.uint8))
     if a.ndim == 1:
-        a = a.reshape(-1, record_bytes(stride))
+        a = a.reshape(-1, pose_record_bytes(stride) if pose else record_bytes(stride))
     n = a.shape[0]
     hdr = a[:, :64].copy().view(np.int32).reshape(n, 16)
     body = a[:, 64:64 + 6 * stride].copy().view(np.uint16).reshape(n, 3, stride)
-    return {"n_matches": hdr[:, 0], "best_h": hdr[:, 1], "inliers": hdr[:, 2], "pair_id": hdr[:, 3],
-            "R": hdr[:, 4:13].copy().view(np.float32).reshape(n, 3, 3), "t": hdr[:, 13:16].copy().view(np.float32).reshape(n, 3),
-            "q": body[:, 0], "t_idx": body[:, 1], "d": body[:, 2], "inlier": a[:, 64 + 6 * stride:64 + 7 * stride]}
+    out = {"n_matches": hdr[:, 0], "best_h": hdr[:, 1], "inliers": hdr[:, 2], "pair_id": hdr[:, 3],
+           "R": hdr[:, 4:13].copy().view(np.float32).reshape(n, 3, 3), "t": hdr[:, 13:16].copy().view(np.float32).reshape(n, 3),
+           "q": body[:, 0], "t_idx": body[:, 1], "d": body[:, 2], "inlier": a[:, 64 + 6 * stride:64 + 7 * stride]}
+    if pose:
+        from .robust_pose import POSE_RESULT_BYTES, decode_results
+
+        rb = record_bytes(stride)
+        if a.shape[1] < pose_record_bytes(stride):
+            raise ValueError(f"pose records of stride {stride} are {pose_record_bytes(stride)} bytes, got {a.shape[1]}")
+        out["robust"] = decode_results(a[:, rb:rb + POSE_RESULT_BYTES].copy())
+    return out
 
 
 def rank_pairs(score, k: int, *, ids=None, sel_count=None, stride: int = 0, with_ids: bool = False):
@@ -539,12 +560,16 @@ class HomographyRansac:
     def __init__(self):
         self._lib = _capi.load_library()
 
-    def hypotheses(self, corr, c_off, c_count, n_pairs: int, H: int, *, samples=None, seed: int = 0, return_samples: bool = False):
+    def hypotheses(self, corr, c_off, c_count, n_pairs: int, H: int, *, samples=None, seed: int = 0, return_samples: bool = False,
+                   pair_ids=None, pair_id0: int = 0):
+        """pair_ids (device int32 [n_pairs]) / pair_id0: the pairs' GLOBAL ids, as in EssentialRansac.hypotheses: the
+        device 4-sample stream is keyed by (seed, id, h), so a pair draws the same samples in any batch position."""
         torch = _capi.require_cuda()
         Hm = torch.empty((max(n_pairs, 1), max(H, 1), 9), dtype=torch.float64, device=corr.device)
         s_out = torch.empty((max(n_pairs, 1), max(H, 1), 4), dtype=torch.int32, device=corr.device) if return_samples else None
         check(self._lib.b2s_homography_dlt_batched(ptr(corr), ptr(c_off), ptr(c_count), n_pairs, H, ptr(samples),
-                                                   C.c_uint64(seed & (2**64 - 1)), ptr(s_out), ptr(Hm), current_stream()))
+                                                   C.c_uint64(seed & (2**64 - 1)), ptr(pair_ids), int(pair_id0), ptr(s_out),
+                                                   ptr(Hm), current_stream()))
         Hm = Hm[:n_pairs, :H]
         return (Hm, s_out[:n_pairs, :H]) if return_samples else Hm
 
@@ -710,16 +735,23 @@ class Frontend:
             after_select=None, before_records=None) -> FrontendResult:
         """records: optional device uint8 [n_pairs, record_bytes(max_matches)] — e.g. this rank's slice of the
         all-gather buffer, or the staging buffer of the step's one device->host copy; the last kernel of the
-        step writes every pair's result record into it (pair ids pair_id0 + p).
+        step writes every pair's result record into it (pair ids pair_id0 + p).  With cfg.robust_pose the records are
+        pose records (pose_record_bytes(max_matches) wide, written by the decision kernel), and pair_id0 also keys both
+        RANSAC samplers, so that a pair's answer does not depend on its batch position.
         after_select / before_records: optional callables run (on the current stream) after the selection kernel and
         before the record kernel — where ShardedFrontend starts and joins the collective of the PREVIOUS batch, so
         that it overlaps the multi-wave RANSAC kernels and never the persistent one-CTA-per-SM Hamming kernel."""
         c = self.cfg
         if c.robust_pose is not None:
-            if records is not None or pair_id0 != 0:
-                raise ValueError("robust_pose does not write result records and takes no pair_id0 offset yet")
             if c.winner_only or c.scoring == "tc":
                 raise ValueError("robust_pose scores with the CUDA-core kernel (scoring='cuda', winner_only=False)")
+            if records is not None:
+                if not c.max_matches:
+                    raise ValueError("records need the compact selection layout (max_matches)")
+                need = pose_record_bytes(c.max_matches)
+                if records.ndim != 2 or records.shape[0] < b.n_pairs or records.shape[-1] < need:
+                    raise _capi.B2SError(f"robust_pose writes pose records: need [{b.n_pairs}, >= {need}] bytes "
+                                         f"(pose_record_bytes({c.max_matches})), got {tuple(records.shape)}")
         keys = self.matcher.knn2(b, need_second=bool(c.use_ratio))
         sel = self.matcher.select(b, keys, use_ratio=c.use_ratio, use_cross=c.use_cross, ratio=c.ratio,
                                   sort_by_distance=True, max_matches=c.max_matches, with_corr=True,
@@ -733,11 +765,10 @@ class Frontend:
                 self.robust = RobustPose()
             out = self.robust.run(sel.corr, sel.c_off, sel.count, b.n_pairs, K, c.robust_pose, samples_e=samples, seed=c.seed,
                                   max_m=sel.stride or b.max_nq, hypotheses=c.hypotheses, precision=c.precision,
-                                  mask_stride=sel.stride)
-            if before_records is not None:
-                before_records()
+                                  mask_stride=sel.stride, pair_id0=pair_id0, records=records, sink_sel=sel,
+                                  before_records=before_records)
             return FrontendResult(keys, sel, out.E, out.counts, out.best_h, out.best_count, out.inlier_mask,
-                                  E_refit=out.E_refit, R=out.R, t=out.t, votes=out.votes, robust=out.results,
+                                  E_refit=out.E_refit, R=out.R, t=out.t, votes=out.votes, records=records, robust=out.results,
                                   robust_mask=out.mask)
         E = self.ransac.hypotheses(sel.corr, sel.c_off, sel.count, b.n_pairs, c.hypotheses,
                                    samples=samples, seed=c.seed, K=K, pair_id0=pair_id0)
@@ -769,16 +800,18 @@ class Frontend:
 class RecordView(dict):
     """The result of a step as the arrays the reference hands back, unpacked lazily from the ONE pinned record
     buffer the step downloaded: count, best_h, best_count (per pair), out_q / out_t / out_d / mask (compact,
-    stride = max_matches), R [P, 3, 3], t [P, 3] (float32; zero unless the step ran with_pose)."""
+    stride = max_matches), R [P, 3, 3], t [P, 3] (float32; zero unless the step ran with_pose).  pose=True (a step with
+    FrontendConfig.robust_pose): also "robust", every pair's b2s_pose_result (robust_pose.POSE_RESULT_DTYPE [P]);
+    best_h / best_count / mask / R / t are then those of the selected model."""
 
-    def __init__(self, host_records, stride: int):
+    def __init__(self, host_records, stride: int, pose: bool = False):
         super().__init__()
-        self.records, self.stride = host_records, stride
+        self.records, self.stride, self.pose = host_records, stride, bool(pose)
 
     def _fill(self):
         import torch
 
-        u = unpack_records(self.records.numpy(), self.stride)
+        u = unpack_records(self.records.numpy(), self.stride, pose=self.pose)
         if (u["n_matches"] < 0).any():     # the selection kernel's overflow flag (a pair larger than the declared maximum / stride)
             raise _capi.B2SError("select kernel: a pair did not fit the declared maximum rows / record stride (count = -1)")
         flat = lambda a: torch.from_numpy(np.ascontiguousarray(a).reshape(-1))
@@ -787,10 +820,16 @@ class RecordView(dict):
                            "out_q": flat(u["q"].astype(np.int32)), "out_t": flat(u["t_idx"].astype(np.int32)),
                            "out_d": flat(u["d"].astype(np.int32)), "mask": flat(u["inlier"].copy()),
                            "R": torch.from_numpy(u["R"].copy()), "t": torch.from_numpy(u["t"].copy())})
+        if self.pose:
+            dict.__setitem__(self, "robust", u["robust"])
 
     def __missing__(self, key):
-        self._fill()
-        return dict.__getitem__(self, key)
+        if not getattr(self, "_filled", False):
+            self._fill()                    # raises (and raises again on the next lookup) for an overflowed pair
+            self._filled = True
+            if dict.__contains__(self, key):
+                return dict.__getitem__(self, key)
+        raise KeyError(key)
 
 
 class SequenceTracker:
@@ -800,10 +839,12 @@ class SequenceTracker:
     Frames (descriptors uint8 [F, N, 32], keypoints float32 [F, N, 2], pinned) are uploaded once each; every
     chunk ends with the record kernel and ONE device->host copy of its records (it was seven copies per chunk).
     ``run`` returns a RecordView over the pinned record buffer.  For several steps in flight use SequencePipeline.
+    K: 3x3 intrinsics of the keypoints (None = identity), passed to every Frontend.run — robust pose at pixel scale
+    needs them (adaptive threshold units, cheirality, decompose_homography).
     """
 
     def __init__(self, n_frames: int, frame_rows: int, cfg: FrontendConfig, variant: int = _capi.VARIANT_I8MMA1,
-                 chunks: int = 4, device=None, use_graph: bool = False):
+                 chunks: int = 4, device=None, use_graph: bool = False, K=None):
         torch = _capi.require_cuda()
         if not cfg.max_matches:
             raise ValueError("SequenceTracker needs max_matches (compact output stride)")
@@ -817,10 +858,11 @@ class SequenceTracker:
         chunks = max(1, min(chunks, self.n_pairs))
         self.bounds = [(self.n_pairs * c // chunks, self.n_pairs * (c + 1) // chunks) for c in range(chunks)]
         self.s_up, self.s_down = torch.cuda.Stream(self.dev), torch.cuda.Stream(self.dev)
-        self.rec_bytes = record_bytes(cfg.max_matches)
+        self.K, self.pose = K, cfg.robust_pose is not None
+        self.rec_bytes = step_record_bytes(cfg)
         self.rec_dev = torch.empty((self.n_pairs, self.rec_bytes), dtype=torch.uint8, device=self.dev)
         self.rec_host = torch.empty((self.n_pairs, self.rec_bytes), dtype=torch.uint8).pin_memory()
-        self.out = RecordView(self.rec_host, cfg.max_matches)
+        self.out = RecordView(self.rec_host, cfg.max_matches, self.pose)
         self._batches = None
         self.h2d_bytes = int(self.F * frame_rows * (DESC_BYTES + 8))
         self.d2h_bytes = int(self.rec_host.numel())
@@ -829,7 +871,7 @@ class SequenceTracker:
 
     def run(self, desc_host, kp_host, counts: np.ndarray):
         """desc_host: pinned uint8 [F*N, 32]; kp_host: pinned float32 [F*N, 2]; counts: rows used per frame."""
-        self.out = RecordView(self.rec_host, self.cfg.max_matches)
+        self.out = RecordView(self.rec_host, self.cfg.max_matches, self.pose)
         if not self.use_graph:
             return self._run_eager(desc_host, kp_host, counts)
         key = (desc_host.data_ptr(), kp_host.data_ptr(), np.asarray(counts).tobytes())
@@ -867,7 +909,7 @@ class SequenceTracker:
                 ups.append(ev)
         for c, (lo, hi) in enumerate(self.bounds):
             main.wait_event(ups[c])
-            res = self.fe.run(self._batches[c], records=self.rec_dev[lo:hi], pair_id0=lo)
+            res = self.fe.run(self._batches[c], K=self.K, records=self.rec_dev[lo:hi], pair_id0=lo)
             done = torch.cuda.Event()
             done.record(main)
             keep.append(res)
@@ -895,10 +937,13 @@ class SequencePipeline:
       run on ONE stream and never interleave; accepts different host buffers on every call without re-capture.
 
     submit() is asynchronous and returns the slot; result(slot) waits for that slot's download and returns a
-    RecordView over its pinned record buffer (valid until the slot is submitted again)."""
+    RecordView over its pinned record buffer (valid until the slot is submitted again).  With cfg.robust_pose the
+    records are pose records (pose_record_bytes per pair) and the view has "robust".  K: 3x3 intrinsics of the
+    keypoints (None = identity), passed to every Frontend.run."""
 
     def __init__(self, n_frames: int, frame_rows: int, cfg: FrontendConfig, variant: int = _capi.VARIANT_I8MMA1,
-                 depth: int = 3, device=None, use_graph: bool = True, schedule: str = "interleaved", after_compute=None):
+                 depth: int = 3, device=None, use_graph: bool = True, schedule: str = "interleaved", after_compute=None,
+                 K=None):
         torch = _capi.require_cuda()
         if not cfg.max_matches:
             raise ValueError("SequencePipeline needs max_matches (compact output stride)")
@@ -912,7 +957,8 @@ class SequencePipeline:
         shared_fe = Frontend(cfg, variant=variant) if schedule == "serial" else None   # one stream: one workspace serves every slot
         self.s_up, self.s_compute, self.s_down = (torch.cuda.Stream(self.dev) for _ in range(3))
         P = self.n_pairs
-        self.rec_bytes = record_bytes(cfg.max_matches)
+        self.K = K
+        self.rec_bytes = step_record_bytes(cfg)
         self.slots = []
         for _ in range(self.depth):
             self.slots.append({
@@ -933,7 +979,7 @@ class SequencePipeline:
 
     # ---- shared -----------------------------------------------------------------------------------------
     def _run_kernels(self, sl):
-        sl["res"] = sl["fe"].run(sl["batch"], records=sl["rec_dev"], pair_id0=0)
+        sl["res"] = sl["fe"].run(sl["batch"], K=self.K, records=sl["rec_dev"], pair_id0=0)
 
     def _after(self, sl):
         # A collective hook runs EAGERLY behind the slot's graph, never inside it: graphs of different slots replay on
@@ -1028,7 +1074,7 @@ class SequencePipeline:
     def result(self, slot: int):
         sl = self.slots[slot]
         sl["downloaded"].synchronize()
-        return RecordView(sl["rec_host"], self.cfg.max_matches)
+        return RecordView(sl["rec_host"], self.cfg.max_matches, self.cfg.robust_pose is not None)
 
     def streams(self):
         if self.schedule == "interleaved":
@@ -1041,18 +1087,19 @@ class PairPipeline:
     high-density pairs, config #4): `depth` steps in flight, each on its own stream — upload of the pairs'
     descriptors and keypoints from pinned host memory, ONE CUDA graph with every kernel of the step, ONE download of
     the result records.  Pair p's query / train rows live at p * rows_q / p * rows_t of the slot's device buffers
-    (fixed stride, so the copies are four contiguous transfers); the per-pair row counts may be ragged."""
+    (fixed stride, so the copies are four contiguous transfers); the per-pair row counts may be ragged.  With
+    cfg.robust_pose the records are pose records; K: 3x3 intrinsics of the keypoints (None = identity)."""
 
     def __init__(self, n_pairs: int, rows_q: int, rows_t: int, cfg: FrontendConfig, variant: int = _capi.VARIANT_I8MMA1,
-                 depth: int = 2, device=None, use_graph: bool = True, after_compute=None):
+                 depth: int = 2, device=None, use_graph: bool = True, after_compute=None, K=None):
         torch = _capi.require_cuda()
         if not cfg.max_matches:
             raise ValueError("PairPipeline needs max_matches (record stride)")
         self.torch, self.cfg = torch, cfg
         self.dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.P, self.rq, self.rt, self.depth = int(n_pairs), int(rows_q), int(rows_t), max(1, depth)
-        self.after_compute, self.use_graph = after_compute, use_graph
-        self.rec_bytes = record_bytes(cfg.max_matches)
+        self.after_compute, self.use_graph, self.K = after_compute, use_graph, K
+        self.rec_bytes = step_record_bytes(cfg)
         P = self.P
         self.slots = []
         for _ in range(self.depth):
@@ -1101,7 +1148,7 @@ class PairPipeline:
                          kp_q=sl["kq"], kp_t=sl["kt"], q_src=pack[2 * P + 2:3 * P + 2], t_src=pack[3 * P + 2:])
 
     def _run_kernels(self, sl):
-        sl["res"] = sl["fe"].run(sl["batch"], records=sl["rec_dev"], pair_id0=0)
+        sl["res"] = sl["fe"].run(sl["batch"], K=self.K, records=sl["rec_dev"], pair_id0=0)
 
     def submit(self, staged) -> int:
         torch = self.torch
@@ -1143,7 +1190,7 @@ class PairPipeline:
     def result(self, slot: int):
         sl = self.slots[slot]
         sl["downloaded"].synchronize()
-        return RecordView(sl["rec_host"], self.cfg.max_matches)
+        return RecordView(sl["rec_host"], self.cfg.max_matches, self.cfg.robust_pose is not None)
 
     def streams(self):
         return tuple(sl["stream"] for sl in self.slots)

@@ -4,8 +4,9 @@ Per pair: the adaptive RANSAC threshold from the median displacement, the essent
 the per-pair threshold, K7 refit + decomposition + cheirality vote), the homography branch (K5 + K6 + selection at
 th = 3, n-point DLT refit, decompose_homography), per-branch inlier ratio / median parallax / cheirality / score, model
 selection and the five stability gates.  The answer is one fixed-size ``b2s_pose_result`` per pair (include/b2s.h)
-plus the selected model's inlier flags in the input's CSR layout.  Everything runs on the current stream: no host
-sync, no allocation after the first call of a shape, capturable in a CUDA graph.
+plus the selected model's inlier flags in the input's CSR layout; given a record buffer, the decision kernel also
+writes every pair's pose record (include/b2s.h: the result record, then the b2s_pose_result).  Everything runs on the
+current stream: no host sync, no allocation after the first call of a shape, capturable in a CUDA graph.
 """
 from __future__ import annotations
 
@@ -23,6 +24,7 @@ ROBUST_POSE_CONFIG_BYTES = 80
 # outcome / method / gate codes of b2s_pose_result
 POSE_ESTIMATE, POSE_GATE_FAILED, POSE_ERR_MATCHES, POSE_ERR_EIGHT, POSE_ERR_ESSENTIAL, POSE_ERR_HOMOGRAPHY, \
     POSE_ERR_TRANSLATION = range(7)
+POSE_EMPTY = -1                   # outcome of a record slot that holds no pair (padding of a sharded gather buffer)
 METHODS = ("essential", "homography")
 GATE_REASONS = (None, "low_inlier_count", "low_inlier_ratio", "low_parallax", "cheirality_inliers", "cheirality_ratio")
 
@@ -183,12 +185,19 @@ class RobustPose:
         return self._cfg_dev, len(host)
 
     def run(self, corr, c_off, c_count, n_pairs: int, K, cfg, samples_e=None, samples_h=None, seed: int = 0, *,
-            max_m: int, hypotheses: int = 2000, precision: int = 64, mask_stride: int = 0) -> RobustPoseOutput:
+            max_m: int, hypotheses: int = 2000, precision: int = 64, mask_stride: int = 0, pair_id0: int = 0,
+            records=None, sink_sel=None, before_records=None) -> RobustPoseOutput:
         """corr: device float32 [rows, 4] (x1, y1, x2, y2); c_off / c_count: device int32 CSR of the pairs; K: 3x3
         intrinsics (None = identity); cfg: RobustPoseConfig (or an object with its fields), or one per pair.
         samples_e [n_pairs, H, 8] / samples_h [n_pairs, H, 4]: host-drawn RANSAC samples (device int32), or None =
         the device sampler with `seed` (essential) and homography_seed(seed).  max_m >= every c_count (host-known);
-        mask_stride: the compact stride when pairs live at p * stride (the unused tails of the masks are cleared)."""
+        mask_stride: the compact stride when pairs live at p * stride (the unused tails of the masks are cleared).
+        pair_id0: global id of pair 0; both device samplers draw from (seed, pair_id0 + p, h), so a pair draws the same
+        samples in whichever batch or shard it is processed.  records (device uint8 [n_pairs, >= pose_record_bytes(S)])
+        with sink_sel (the Selection in the compact layout, S = its stride): the decision kernel writes every pair's
+        pose record, header pair id pair_id0 + p.  before_records: a callable run on the host immediately before the
+        decision kernel is enqueued (ShardedFrontend joins the previous batch's collective there, which reads the buffer
+        the kernel writes)."""
         torch = _capi.require_cuda()
         lib, st, P = self._lib, current_stream(), int(n_pairs)
         dev = corr.device
@@ -205,8 +214,8 @@ class RobustPose:
         check(lib.b2s_displacement_median_batched(c, o, n, None, P, ptr(cfg_d), n_cfg, ptr(b["med_all"]), ptr(b["th"]),
                                                   ptr(b["th2"]), st))
         # 2. essential RANSAC at the per-pair threshold
-        check(lib.b2s_eight_point_batched(c, o, n, P, He, ptr(samples_e), seed64, None, 0, None, ptr(Kd), ptr(Kinv),
-                                          ptr(b["E"]), st))
+        check(lib.b2s_eight_point_batched(c, o, n, P, He, ptr(samples_e), seed64, None, int(pair_id0), None, ptr(Kd),
+                                          ptr(Kinv), ptr(b["E"]), st))
         check(lib.b2s_ransac_score_batched(c, o, n, P, ptr(b["E"]), He, 0.0, ptr(b["th2"]), int(precision), int(max_m),
                                            ptr(b["counts_e"]), st))
         check(lib.b2s_ransac_select(ptr(b["counts_e"]), c, o, n, P, ptr(b["E"]), He, 0.0, ptr(b["th2"]), ptr(b["best_h_e"]),
@@ -220,17 +229,26 @@ class RobustPose:
         check(lib.b2s_displacement_median_batched(c, o, n, ptr(b["mask_e"]), P, None, 0, ptr(b["med_in"]), None, None, st))
         # 4. homography RANSAC at th = 3
         check(lib.b2s_homography_dlt_batched(c, o, n, P, Hh, ptr(samples_h), C.c_uint64(homography_seed(seed)), None,
-                                             ptr(b["Hm"]), st))
+                                             int(pair_id0), None, ptr(b["Hm"]), st))
         check(lib.b2s_homography_score_batched(c, o, n, P, ptr(b["Hm"]), Hh, HOMOGRAPHY_THRESHOLD, None, ptr(b["counts_h"]), st))
         check(lib.b2s_homography_select(ptr(b["counts_h"]), c, o, n, P, ptr(b["Hm"]), Hh, HOMOGRAPHY_THRESHOLD, None,
                                         ptr(b["best_h_h"]), ptr(b["best_c_h"]), ptr(b["mask_h"]), st))
         # 5. n-point DLT on the homography winner's inliers
         check(lib.b2s_refit_homography_batched(c, o, n, ptr(b["mask_h"]), P, ptr(b["H_fit"]), ptr(b["h_used"]), st))
-        # 6. decomposition, diagnostics, selection, gates
-        check(lib.b2s_robust_pose_decide(o, n, P, ptr(b["best_h_e"]), ptr(b["best_c_e"]), ptr(b["mask_e"]), ptr(b["R"]),
-                                         ptr(b["t"]), ptr(b["votes"]), ptr(b["med_in"]), ptr(b["med_all"]), ptr(b["th"]),
-                                         ptr(b["best_h_h"]), ptr(b["best_c_h"]), ptr(b["mask_h"]), ptr(b["H_fit"]), ptr(Kinv),
-                                         ptr(cfg_d), n_cfg, ptr(b["results"]), ptr(b["mask"]), int(mask_stride), st))
+        # 6. decomposition, diagnostics, selection, gates (+ the pose records)
+        sink = None
+        if records is not None:
+            if sink_sel is None or not sink_sel.stride:
+                raise ValueError("pose records need the selection in the compact layout (sink_sel with a stride)")
+            sink = _capi.RecordSink(records.data_ptr(), int(records.shape[-1]), sink_sel.out_q.data_ptr(),
+                                    sink_sel.out_t.data_ptr(), sink_sel.out_d.data_ptr(), int(sink_sel.stride), int(pair_id0))
+        if before_records is not None:
+            before_records()
+        check(lib.b2s_robust_pose_decide_records(
+            o, n, P, ptr(b["best_h_e"]), ptr(b["best_c_e"]), ptr(b["mask_e"]), ptr(b["R"]), ptr(b["t"]), ptr(b["votes"]),
+            ptr(b["med_in"]), ptr(b["med_all"]), ptr(b["th"]), ptr(b["best_h_h"]), ptr(b["best_c_h"]), ptr(b["mask_h"]),
+            ptr(b["H_fit"]), ptr(Kinv), ptr(cfg_d), n_cfg, ptr(b["results"]), ptr(b["mask"]), int(mask_stride),
+            C.byref(sink) if sink is not None else None, st))
         rows = int(corr.shape[0])
         return RobustPoseOutput(
             results=b["results"][:P], mask=b["mask"][:rows], packed=b["packed"][:P * POSE_RESULT_BYTES + rows] if P else b["packed"][:0],

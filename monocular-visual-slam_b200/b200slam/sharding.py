@@ -126,6 +126,17 @@ class RecordGather:
         return torch.cat(parts, dim=0)
 
 
+def _mark_empty(rows, cfg):
+    """Records [n, record_bytes] that hold no pair (padding slots of a short shard): pair id -1, and in pose records
+    outcome -1 (robust_pose.POSE_EMPTY), so that an empty slot never decodes as an estimate."""
+    from .frontend import record_bytes
+
+    rows[:, 12:16] = 0xFF                                              # int32 header[3] = -1
+    if cfg.robust_pose is not None:
+        o = record_bytes(cfg.max_matches)                              # the pose block: b2s_pose_result.outcome
+        rows[:, o:o + 4] = 0xFF
+
+
 DEFAULT_LANES = 3    # measured on the metric's step (tools/lanes_ab.py): 1 lane 473.5 k pairs/s, 2 lanes 488.7 k, 3 lanes 494.8 k
 
 
@@ -158,12 +169,12 @@ class ShardedFrontend:
         import os
 
         from . import _capi
-        from .frontend import Frontend, record_bytes
+        from .frontend import Frontend, step_record_bytes
 
         torch = _capi.require_cuda()
         if not cfg.max_matches:
             raise ValueError("ShardedFrontend needs max_matches (record stride)")
-        self.cfg = cfg            # cfg.with_pose decides whether the records carry R | t (else zeros)
+        self.cfg = cfg            # cfg.with_pose decides whether the records carry R | t (else zeros); cfg.robust_pose: pose records
         self.dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         # lanes: the launch sets of a batch alternate between `lanes` streams (each with its own Frontend = its own
         # workspaces), so the tail of one set's kernels, its one-CTA-per-pair selection / winner kernels and the gaps
@@ -173,7 +184,7 @@ class ShardedFrontend:
         self.fes = [Frontend(self.cfg, variant=_capi.VARIANT_I8MMA1 if variant is None else variant) for _ in range(self.lanes)]
         self.fe = self.fes[0]
         self._side = [torch.cuda.Stream(device=self.dev) for _ in range(self.lanes - 1)]
-        self.rec_bytes = record_bytes(cfg.max_matches)
+        self.rec_bytes = step_record_bytes(cfg)      # pose records when cfg.robust_pose is set
         self.sets = max(1, int(sets_per_gather))
         self.n_pairs_global = int(n_pairs_global)
         self.world, self.group = _world(group), group
@@ -182,11 +193,11 @@ class ShardedFrontend:
         # the last gathered batch [world][sets * cap][record]
         self.gather = RecordGather(self.world * self.sets * self.cap, self.rec_bytes, dtype=torch.uint8, device=self.dev, group=group)
         self.rank = self.gather.rank
-        self.gather.buf.view(torch.int32).reshape(self.world, self.gather.cap, -1)[:, :, 3] = -1   # padding slots: pair id -1
+        _mark_empty(self.gather.buf.view(-1, self.rec_bytes), cfg)     # padding slots: pair id -1
         self.pipelined = bool(pipelined) and os.environ.get("B2S_GATHER", "pipelined") != "sync"
         if self.pipelined and self.world > 1:
             self.send = torch.zeros((self.sets * self.cap, self.rec_bytes), dtype=torch.uint8, device=self.dev)
-            self.send.view(torch.int32)[:, 3] = -1
+            _mark_empty(self.send, cfg)
         else:
             self.send = self.gather.local               # in-place: the send slice of the gather buffer itself
         self.lo, self.hi = shard_bounds(self.n_pairs_global, self.rank, self.world)

@@ -13,6 +13,15 @@
 
 namespace b2s {
 
+// ---- result records (include/b2s.h) -------------------------------------------
+// record = 16 x int32 header | S x u16 queryIdx | S x u16 trainIdx | S x u16 distance | S x u8 inlier | pad to 64 B
+__host__ __device__ constexpr size_t record_bytes(int S) { return ((size_t)64 + 7 * (size_t)S + 63) & ~(size_t)63; }
+// pose record = record | b2s_pose_result | zero pad to B2S_POSE_BLOCK_BYTES; the pose block starts on a 64-byte
+// boundary, so its doubles are aligned
+__host__ __device__ constexpr size_t pose_record_bytes(int S) { return record_bytes(S) + B2S_POSE_BLOCK_BYTES; }
+static_assert(record_bytes(1) == 128 && record_bytes(500) == 3584 && pose_record_bytes(500) == 3840, "record layout");
+static_assert(B2S_POSE_BLOCK_BYTES - B2S_POSE_RESULT_BYTES == 56, "pose block = b2s_pose_result + 56 zero bytes");
+
 // ---- error plumbing (no exceptions across the C ABI) --------------------------
 void set_error(const char* fmt, ...);
 int cuda_fail(cudaError_t e, const char* what);

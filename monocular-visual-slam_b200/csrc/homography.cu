@@ -49,7 +49,8 @@ __device__ __forceinline__ bool transfer_inlier(const double (&h)[9], const doub
 // ---- K5: 4-point DLT, one thread per hypothesis ----------------------------------------
 __global__ void __launch_bounds__(kHomThreads) homography_dlt_kernel(
     const float4* __restrict__ corr, const int32_t* __restrict__ c_off, const int32_t* __restrict__ c_count, int H,
-    const int32_t* __restrict__ samples_in, uint64_t seed, int32_t* __restrict__ samples_out, double* __restrict__ H_out) {
+    const int32_t* __restrict__ samples_in, uint64_t seed, const int32_t* __restrict__ pair_ids, int pair_id0,
+    int32_t* __restrict__ samples_out, double* __restrict__ H_out) {
   const int pair = blockIdx.y;
   const int h = blockIdx.x * blockDim.x + threadIdx.x;
   if (h >= H) return;
@@ -60,7 +61,7 @@ __global__ void __launch_bounds__(kHomThreads) homography_dlt_kernel(
   if (samples_in) {
     for (int k = 0; k < 4; ++k) idx[k] = samples_in[((size_t)pair * H + h) * 4 + k];
   } else if (M >= 4) {
-    draw_distinct<4>(seed, pair, h, M, idx);
+    draw_distinct<4>(seed, pair_ids ? pair_ids[pair] : pair_id0 + pair, h, M, idx);   // keyed by the GLOBAL pair id
   } else {
     for (int k = 0; k < 4; ++k) idx[k] = 0;
   }
@@ -225,7 +226,8 @@ __global__ void __launch_bounds__(256) homography_select_kernel(
 extern "C" {
 
 int b2s_homography_dlt_batched(const float* corr, const int32_t* c_off, const int32_t* c_count, int n_pairs, int H,
-                               const int32_t* samples_in, uint64_t seed, int32_t* samples_out, double* H_out, void* stream) {
+                               const int32_t* samples_in, uint64_t seed, const int32_t* pair_ids, int pair_id0,
+                               int32_t* samples_out, double* H_out, void* stream) {
   using namespace b2s;
   B2S_REQUIRE(corr && c_off && c_count && H_out, "null pointer");
   B2S_REQUIRE(n_pairs >= 0 && H >= 0, "negative size");
@@ -233,7 +235,7 @@ int b2s_homography_dlt_batched(const float* corr, const int32_t* c_off, const in
   if (n_pairs == 0 || H == 0) return B2S_OK;
   dim3 grid((H + kHomThreads - 1) / kHomThreads, n_pairs);
   homography_dlt_kernel<<<grid, kHomThreads, 0, static_cast<cudaStream_t>(stream)>>>(
-      reinterpret_cast<const float4*>(corr), c_off, c_count, H, samples_in, seed, samples_out, H_out);
+      reinterpret_cast<const float4*>(corr), c_off, c_count, H, samples_in, seed, pair_ids, pair_id0, samples_out, H_out);
   B2S_CUDA(cudaGetLastError());
   note_launch();
   return B2S_OK;

@@ -17,8 +17,7 @@
 
 namespace b2s {
 
-// record = 16 x int32 header | S x u16 queryIdx | S x u16 trainIdx | S x u16 distance | S x u8 inlier | pad to 64 B
-__host__ __device__ inline size_t record_bytes(int S) { return ((size_t)64 + 7 * (size_t)S + 63) & ~(size_t)63; }
+// record layout: record_bytes / pose_record_bytes (common.cuh)
 
 struct PackParams {
   const int32_t* __restrict__ count;
@@ -145,6 +144,7 @@ __global__ void __launch_bounds__(1024) rank_pairs_kernel(const int32_t* __restr
 extern "C" {
 
 size_t b2s_record_bytes(int max_matches) { return b2s::record_bytes(max_matches); }
+size_t b2s_pose_record_bytes(int max_matches) { return b2s::pose_record_bytes(max_matches); }
 
 int b2s_pack_records(const int32_t* count, const int32_t* count_total, const int32_t* best_h, const int32_t* best_count, const int32_t* out_q,
                      const int32_t* out_t, const int32_t* out_d, const uint8_t* inlier_mask, const double* R,

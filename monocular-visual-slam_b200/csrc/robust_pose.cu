@@ -9,7 +9,7 @@
 //   * refit_homography_kernel: one CTA per pair, the structure of refit_essential_kernel (pose.cu): fixed-order
 //     reductions, the 9x9 Gram matrix of the DLT rows in float64, warp-cooperative parallel-order Jacobi.
 //   * robust_pose_decide_kernel: one CTA per pair; lane 0 makes the decision, the CTA writes the selected
-//     model's inlier flags.
+//     model's inlier flags and, given a record sink, the pair's pose record (include/b2s.h).
 #include "common.cuh"
 
 namespace b2s {
@@ -367,7 +367,7 @@ __global__ void __launch_bounds__(kDecideThreads) robust_pose_decide_kernel(
     const float* __restrict__ all_median, const double* __restrict__ th, const int32_t* __restrict__ h_best_h,
     const int32_t* __restrict__ h_inliers, const uint8_t* __restrict__ h_mask, const double* __restrict__ H_fit,
     const Mat3Arg Kinv, const b2s_robust_pose_config* __restrict__ cfg, int n_cfg,
-    b2s_pose_result* __restrict__ results, uint8_t* __restrict__ out_mask, int mask_stride) {
+    b2s_pose_result* __restrict__ results, uint8_t* __restrict__ out_mask, int mask_stride, const b2s_record_sink sink) {
   __shared__ int s_src;   // 0: essential mask, 1: homography mask, -1: zeros
   const int pair = blockIdx.x, tid = threadIdx.x;
   const int M = max(c_count[pair], 0);
@@ -455,6 +455,42 @@ __global__ void __launch_bounds__(kDecideThreads) robust_pose_decide_kernel(
   const int off = c_off[pair];
   for (int m = tid; m < M; m += kDecideThreads) out_mask[off + m] = from ? from[off + m] : (uint8_t)0;
   for (int m = M + tid; m < mask_stride; m += kDecideThreads) out_mask[off + m] = 0;   // unused tail of a compact slot
+  if (!sink.records) return;
+  // The pair's pose record, written by the kernel that holds the answer (no extra launch at the end of the step): this
+  // is the send slice of the all-gather / the source of the step's one device->host copy.  The result is read back
+  // from `results` (written by thread 0 before the barrier), so the decision keeps its registers.
+  uint8_t* rec = sink.records + (size_t)pair * sink.record_bytes;
+  const int S = sink.stride, n = min(M, S);
+  const b2s_pose_result* r = results + pair;
+  if (tid < 16) {
+    const int outcome = r->outcome;
+    const bool answer = outcome == B2S_POSE_ESTIMATE || outcome == B2S_POSE_GATE_FAILED;
+    int32_t v;
+    if (tid == 0) v = c_count[pair];                   // the selection count (-1 on overflow)
+    else if (tid == 1) v = answer ? (r->method == B2S_POSE_METHOD_HOMOGRAPHY ? r->h_best_h : r->e_best_h) : -1;
+    else if (tid == 2) v = r->inliers;
+    else if (tid == 3) v = sink.pair_id0 + pair;
+    else if (tid < 13) v = __float_as_int((float)r->R[tid - 4]);   // zero for an error outcome
+    else v = __float_as_int((float)r->t[tid - 13]);
+    reinterpret_cast<int32_t*>(rec)[tid] = v;
+  } else if (tid < 16 + B2S_POSE_BLOCK_BYTES / 8) {    // pose block: the 200-byte result, then 56 zero bytes
+    const int w = tid - 16;
+    reinterpret_cast<uint64_t*>(rec + record_bytes(S))[w] =
+        w < B2S_POSE_RESULT_BYTES / 8 ? reinterpret_cast<const uint64_t*>(r)[w] : 0ull;
+  }
+  uint16_t* rq = reinterpret_cast<uint16_t*>(rec + 64);
+  uint16_t* rt = rq + S;
+  uint16_t* rd = rt + S;
+  uint8_t* rm = reinterpret_cast<uint8_t*>(rd + S);
+  const size_t base = (size_t)pair * S;
+  for (int k = tid; k < S; k += kDecideThreads) {
+    const bool live = k < n;
+    rq[k] = live ? (uint16_t)sink.out_q[base + k] : (uint16_t)0;
+    rt[k] = live ? (uint16_t)sink.out_t[base + k] : (uint16_t)0;
+    rd[k] = live ? (uint16_t)sink.out_d[base + k] : (uint16_t)0;
+    rm[k] = (live && from) ? from[off + k] : (uint8_t)0;
+  }
+  for (size_t k = 64 + 7 * (size_t)S + tid; k < record_bytes(S); k += kDecideThreads) rec[k] = 0;   // every byte is defined
 }
 
 }  // namespace b2s
@@ -489,26 +525,59 @@ int b2s_refit_homography_batched(const float* corr, const int32_t* c_off, const 
   return B2S_OK;
 }
 
+static int robust_pose_decide(const int32_t* c_off, const int32_t* c_count, int n_pairs, const int32_t* e_best_h,
+                              const int32_t* e_inliers, const uint8_t* e_mask, const double* e_R, const double* e_t,
+                              const int32_t* e_votes, const float* e_median, const float* all_median, const double* th,
+                              const int32_t* h_best_h, const int32_t* h_inliers, const uint8_t* h_mask, const double* H_fit,
+                              const double* Kinv_host, const b2s_robust_pose_config* cfg, int n_cfg,
+                              b2s_pose_result* results, uint8_t* out_mask, int mask_stride, const b2s_record_sink* sink,
+                              void* stream) {
+  using namespace b2s;
+  B2S_REQUIRE(c_off && c_count && e_best_h && e_inliers && e_mask && e_R && e_t && e_votes && e_median && all_median && th &&
+                  h_best_h && h_inliers && h_mask && H_fit && cfg && results && out_mask, "null pointer");
+  B2S_REQUIRE(n_pairs >= 0, "negative size");
+  B2S_REQUIRE(n_cfg == 1 || n_cfg == n_pairs, "n_cfg must be 1 or n_pairs");
+  b2s_record_sink sk{};
+  if (sink && sink->records) {
+    B2S_REQUIRE(sink->out_q && sink->out_t && sink->out_d && sink->stride > 0, "record sink: selection outputs and stride required");
+    B2S_REQUIRE(sink->record_bytes >= pose_record_bytes(sink->stride) && (sink->record_bytes & 15u) == 0 &&
+                    ((uintptr_t)sink->records & 15u) == 0,
+                "record sink: record_bytes (%zu) must be >= b2s_pose_record_bytes(stride) = %zu and 16-byte aligned",
+                sink->record_bytes, pose_record_bytes(sink->stride));
+    sk = *sink;
+  }
+  if (n_pairs == 0) return B2S_OK;
+  Mat3Arg Kinv;
+  for (int i = 0; i < 9; ++i) Kinv.m[i] = Kinv_host ? Kinv_host[i] : ((i % 4 == 0) ? 1.0 : 0.0);
+  robust_pose_decide_kernel<<<n_pairs, kDecideThreads, 0, static_cast<cudaStream_t>(stream)>>>(
+      c_off, c_count, e_best_h, e_inliers, e_mask, e_R, e_t, e_votes, e_median, all_median, th, h_best_h, h_inliers,
+      h_mask, H_fit, Kinv, cfg, n_cfg, results, out_mask, mask_stride, sk);
+  B2S_CUDA(cudaGetLastError());
+  note_launch();
+  return B2S_OK;
+}
+
 int b2s_robust_pose_decide(const int32_t* c_off, const int32_t* c_count, int n_pairs, const int32_t* e_best_h,
                            const int32_t* e_inliers, const uint8_t* e_mask, const double* e_R, const double* e_t,
                            const int32_t* e_votes, const float* e_median, const float* all_median, const double* th,
                            const int32_t* h_best_h, const int32_t* h_inliers, const uint8_t* h_mask, const double* H_fit,
                            const double* Kinv_host, const b2s_robust_pose_config* cfg, int n_cfg,
                            b2s_pose_result* results, uint8_t* out_mask, int mask_stride, void* stream) {
-  using namespace b2s;
-  B2S_REQUIRE(c_off && c_count && e_best_h && e_inliers && e_mask && e_R && e_t && e_votes && e_median && all_median && th &&
-                  h_best_h && h_inliers && h_mask && H_fit && cfg && results && out_mask, "null pointer");
-  B2S_REQUIRE(n_pairs >= 0, "negative size");
-  B2S_REQUIRE(n_cfg == 1 || n_cfg == n_pairs, "n_cfg must be 1 or n_pairs");
-  if (n_pairs == 0) return B2S_OK;
-  Mat3Arg Kinv;
-  for (int i = 0; i < 9; ++i) Kinv.m[i] = Kinv_host ? Kinv_host[i] : ((i % 4 == 0) ? 1.0 : 0.0);
-  robust_pose_decide_kernel<<<n_pairs, kDecideThreads, 0, static_cast<cudaStream_t>(stream)>>>(
-      c_off, c_count, e_best_h, e_inliers, e_mask, e_R, e_t, e_votes, e_median, all_median, th, h_best_h, h_inliers,
-      h_mask, H_fit, Kinv, cfg, n_cfg, results, out_mask, mask_stride);
-  B2S_CUDA(cudaGetLastError());
-  note_launch();
-  return B2S_OK;
+  return robust_pose_decide(c_off, c_count, n_pairs, e_best_h, e_inliers, e_mask, e_R, e_t, e_votes, e_median, all_median, th,
+                            h_best_h, h_inliers, h_mask, H_fit, Kinv_host, cfg, n_cfg, results, out_mask, mask_stride, nullptr,
+                            stream);
+}
+
+int b2s_robust_pose_decide_records(const int32_t* c_off, const int32_t* c_count, int n_pairs, const int32_t* e_best_h,
+                                   const int32_t* e_inliers, const uint8_t* e_mask, const double* e_R, const double* e_t,
+                                   const int32_t* e_votes, const float* e_median, const float* all_median, const double* th,
+                                   const int32_t* h_best_h, const int32_t* h_inliers, const uint8_t* h_mask,
+                                   const double* H_fit, const double* Kinv_host, const b2s_robust_pose_config* cfg, int n_cfg,
+                                   b2s_pose_result* results, uint8_t* out_mask, int mask_stride, const b2s_record_sink* sink,
+                                   void* stream) {
+  return robust_pose_decide(c_off, c_count, n_pairs, e_best_h, e_inliers, e_mask, e_R, e_t, e_votes, e_median, all_median, th,
+                            h_best_h, h_inliers, h_mask, H_fit, Kinv_host, cfg, n_cfg, results, out_mask, mask_stride, sink,
+                            stream);
 }
 
 }  // extern "C"

@@ -1,7 +1,9 @@
 """World-size-independence check of the sharded library paths (run plain for world 1, or under torchrun):
 writes the gathered result records of a small config #3 batch (pair-sharded ShardedFrontend) or a small
 config #5 sweep (keyframe-sharded ShardedSweep) to --out on rank 0.  tests/test_gpu_records.py compares the
-world-1 and world-2 files bit for bit."""
+world-1 and world-2 files bit for bit.  --robust (configs 2 and 3): the step runs RobustPoseEstimator.estimate_pose
+for every pair (FrontendConfig.robust_pose) and the gathered records are pose records; the output then also holds
+every pair's b2s_pose_result bytes ("robust"); tests/test_gpu_robust_records.py compares those files."""
 import argparse
 import faulthandler
 import json
@@ -16,6 +18,7 @@ import torch
 import torch.distributed as dist
 
 from b200slam.frontend import FrontendConfig, PairBatch, unpack_records
+from b200slam.robust_pose import RobustPoseConfig
 from b200slam.sharding import ShardedFrontend, ShardedSweep, shard_bounds
 from b200slam.synthetic import tracking_pairs
 
@@ -24,14 +27,27 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--config", type=int, default=3)
 ap.add_argument("--out", required=True)
 ap.add_argument("--no-graph-collective", action="store_true", help="keep the collective out of the CUDA graph (diagnostics)")
+ap.add_argument("--robust", action="store_true", help="configs 2 / 3 with robust_pose=RobustPoseConfig(): pose records")
 a = ap.parse_args()
+if a.robust and a.config not in (2, 3):
+    ap.error("--robust applies to the pair-sharded configs 2 and 3")
 rank, world, local = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1)), int(os.environ.get("LOCAL_RANK", 0))
 torch.cuda.set_device(local)
 if world > 1:
     os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 S = 200
-cfg = FrontendConfig(hypotheses=256, max_matches=S, threshold=0.01, seed=99, with_pose=True)
+cfg = FrontendConfig(hypotheses=256, max_matches=S, threshold=0.01, seed=99, with_pose=not a.robust,
+                     robust_pose=RobustPoseConfig() if a.robust else None)
+
+
+def unpack(rec):
+    u = unpack_records(rec, S, pose=a.robust)
+    if a.robust:
+        u["robust"] = u["robust"].view(np.uint8).reshape(len(rec), -1)     # raw bytes: compared bit for bit
+    return u
+
+
 out = {}
 in_graph = None
 sf = sw = None
@@ -48,7 +64,7 @@ if a.config == 3:
         sf.replay()
     sf.flush()
     torch.cuda.synchronize()
-    u = unpack_records(sf.records()[0].cpu().numpy(), S)
+    u = unpack(sf.records()[0].cpu().numpy())
     out = {k: v for k, v in u.items()}
 elif a.config == 2:
     # a batch of 5 launch sets (alternating over the stream lanes), ONE pipelined collective per batch
@@ -67,7 +83,7 @@ elif a.config == 2:
     torch.cuda.synchronize()
     rec = sf.records().cpu().numpy()
     for j in range(sets):
-        for k, v in unpack_records(rec[j], S).items():
+        for k, v in unpack(rec[j]).items():
             out[f"set{j}/{k}"] = v
     out["n_matches"], out["inliers"], out["pair_id"] = out["set0/n_matches"], out["set0/inliers"], out["set0/pair_id"]
 else:
@@ -106,7 +122,7 @@ else:
     out = dict(cand, counts=counts)
 if rank == 0:
     np.savez(a.out, **out)
-    print(json.dumps({"world": world, "config": a.config, "collective_in_graph": in_graph,
+    print(json.dumps({"world": world, "config": a.config, "robust": a.robust, "collective_in_graph": in_graph,
                       "summary": {k: np.asarray(v).reshape(-1)[:5].tolist() for k, v in out.items() if k in ("n_matches", "inliers", "pair_id", "counts")}}))
 sf = sw = None          # graphs that captured the collective go before their communicator
 if world > 1:
